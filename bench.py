@@ -2,6 +2,7 @@
 """Benchmark of the mastering DSP chain (BASELINE.json metric: audio-seconds mastered per wall-second).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]                      # this build, N GPUs of one node
+  python bench.py ... --dump-outputs DIR                                    # + the last timed step's output as DIR/*.npy
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...                                      # the reference's CPU path
 
@@ -16,6 +17,8 @@ compressor + BS.1770 loudness + gain) over the rank's tracks.
   roofline : per kernel from a SERIALISED pass (a one-slot plan: waves follow each other on one stream, so the kernel
              times add up to the step), DRAM traffic per launch from the tracked ncu export under profiles/.
   parity_check : three tracks of the timed batch mastered by the CPU oracle, outside the timed region.
+  --dump-outputs : the mastered audio of the last timed step (rank 0's tracks at a fixed, seeded sample of frame
+             positions, see dump_outputs), so that two builds can be compared output for output on identical inputs.
   time_sharded : (N > 1) BASELINE config C3 - one 60 min 96 kHz track split BY TIME over the N GPUs, halo hand-off
              between neighbours + ONE NCCL all-reduce of the int64[1000] loudness histogram - timed on the device and
              compared bit for bit with the single-plan result.
@@ -42,6 +45,7 @@ KERNEL_ALG_BYTES = {   # per-kernel algorithmic bytes per frame it processes (DE
     "k_kweight_energy": 4, "k_apply_gain": 8}
 ALL_TRACK_KERNELS = ("k_eq", "k_kweight_energy", "k_apply_gain", "k_limiter", "k_true_peak")   # the others see multiband tracks only
 NCU_CSV = os.path.join(ROOT, "profiles", "r02", "ncu_kernels.csv")
+DUMP_VALUES = 8 << 20  # int16 samples --dump-outputs keeps (stored as float32: 32 MB)
 
 
 def parse():
@@ -78,7 +82,14 @@ def parse():
     ap.add_argument("--true-peak", action="store_true", help="also measure the BS.1770 true peak")
     ap.add_argument("--ablate", default="", help="experiments only (profiles/r02/ablation.txt): comma list of "
                     "nomb (no track multiband), allmb, noeq (EQ preset None, no warmth, width 1), nolufs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write the mastered audio of the last timed step "
+                    "(a seeded sample of frames of every track of rank 0) as DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -208,6 +219,23 @@ def fill_batch(torch, synth, d_in, ids, n, secs, fs, dev, block=32):
             view[k + j, :n] = synth.torch_track_batch(1, secs, fs, dev, first_track_id=t)[0]
 
 
+def dump_outputs(path, torch, np, d_out, offsets, n, ids):
+    """What a caller of master_device receives, the packed int16 output, sampled: every track at the same frame
+    positions (all n when they fit in DUMP_VALUES, else a sorted draw of a fixed-seed generator), values as float32.
+      output.npy          [tracks, frames, 2]  float32, the int16 samples
+      output_frame.npy    [frames]             float64, frame position within each track
+      output_track_id.npy [tracks]             float64, the synthetic track id (input seed) of each row"""
+    k = min(n, DUMP_VALUES // (2 * len(offsets)))
+    frames = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    dev = d_out.device
+    idx = torch.tensor(offsets, dtype=torch.int64, device=dev)[:, None] + torch.from_numpy(frames).to(dev)[None, :]
+    out = d_out[idx.reshape(-1)].reshape(len(offsets), k, 2).float().cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "output.npy"), out)
+    np.save(os.path.join(path, "output_frame.npy"), frames.astype(np.float64))
+    np.save(os.path.join(path, "output_track_id.npy"), np.asarray(ids, dtype=np.float64))
+
+
 def run_time_sharded(args, torch, dist, rank, world, dev):
     """BASELINE config C3 through sharding.time_sharded_step: one long 96 kHz track split by time over the ranks."""
     from audio_mastering_engine_b200 import synth, sharding, MasterPlan
@@ -332,6 +360,8 @@ def run_b200(args, rank, world, local_rank):
     barrier()
     clocks = sampler.finish()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, np, d_out, plan.offsets, n, ids)
     launches = plan.launch_count * args.steps
     ms_max = allmax(ms)
     audio_total = total_tracks * secs

@@ -16,10 +16,8 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    import json
-    import numpy as np
     gdir = os.path.join(ROOT, "tests", "golden")
-    arrays = np.load(os.path.join(gdir, "reference_chain.npz"))
-    with open(os.path.join(gdir, "reference_chain.json")) as fh:
-        meta = json.load(fh)
-    return arrays, meta
+    if gdir not in sys.path:
+        sys.path.insert(0, gdir)
+    import make_golden
+    return make_golden.load()

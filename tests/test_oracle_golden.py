@@ -6,7 +6,7 @@ from oracle import chain
 
 
 def test_converters(golden):
-    g, _ = golden
+    g = golden
     assert np.array_equal(chain.to_float(g["conv_in"]), g["conv_float"])
     assert np.array_equal(chain.to_pcm(g["conv_ramp_f32"]), g["conv_ramp_pcm_f32"])
     assert np.array_equal(chain.to_pcm(g["conv_ramp_f32"].astype(np.float64) * 0.999), g["conv_ramp_pcm_f64"])
@@ -15,28 +15,27 @@ def test_converters(golden):
 
 
 def test_chunk_cases_bit_exact(golden):
-    g, meta = golden
-    assert len(meta["cases"]) >= 30
-    for c in meta["cases"]:
+    g = golden
+    assert len(g.cases) >= 30
+    for c in g.cases:
         key, fs, settings = c["key"], c["fs"], c["settings"]
         taps = {}
-        out = chain.process_chunk(g[key + "_in"], fs, settings, taps=taps,
+        out = chain.process_chunk(g.input(c), fs, settings, taps=taps,
                                   compress=chain.compress_dynamic_range_py)
-        assert np.array_equal(taps["warmth"], g[key + "_warmth"]), key
+        assert g.equals(c, "warmth", taps["warmth"]), key
         assert taps["eq"].dtype == np.float32
-        assert np.array_equal(taps["eq"], g[key + "_eq"]), key
-        assert np.array_equal(taps["pre_multiband"], g[key + "_pre_multiband"]), key
-        assert np.array_equal(out, g[key + "_out"]), key
+        assert g.equals(c, "eq", taps["eq"]), key
+        assert g.equals(c, "pre_multiband", taps["pre_multiband"]), key
+        assert g.equals(c, "out", out), key
 
 
 def test_warmth_closed_form_matches_axis_quirk(golden):
     """lfilter(axis=-1) on an (N,2) array == the per-frame 2x2 lower-triangular mix the kernel uses."""
-    g, meta = golden
-    for c in meta["cases"]:
+    g = golden
+    for c in g.cases:
         pct = c["settings"].get("analog_character", 0)
         if pct > 0:
-            x = g[c["key"] + "_in"]
-            assert np.array_equal(chain.warmth_closed_form(x, c["fs"], pct), g[c["key"] + "_warmth"]), c["key"]
+            assert g.equals(c, "warmth", chain.warmth_closed_form(g.input(c), c["fs"], pct)), c["key"]
 
 
 def test_cut_shelf_is_bare_filter():
