@@ -6,7 +6,8 @@ import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = [os.path.join(HERE, "csrc", "ame.cu")]
-DEPS = SRC + [os.path.join(HERE, "csrc", "ame_kernels.cuh"), os.path.join(os.path.dirname(HERE), "include", "ame.h")]
+DEPS = SRC + [os.path.join(HERE, "csrc", "ame_kernels.cuh"), os.path.join(HERE, "csrc", "ame_layout.h"),
+              os.path.join(os.path.dirname(HERE), "include", "ame.h")]
 OUT = os.path.join(HERE, "libame.so")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

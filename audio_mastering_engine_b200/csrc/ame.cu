@@ -3,13 +3,9 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
-#include <cstring>
 #include <dlfcn.h>
-#include <map>
 #include <mutex>
 #include <string>
-#include <tuple>
 #include <vector>
 
 #include "ame_kernels.cuh"
@@ -36,8 +32,6 @@ int fail(int code, const char *fmt, ...) {
         if (e_ != cudaSuccess)                                                                     \
             return fail(AME_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
     } while (0)
-
-inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
 
 // Every entry point works on its plan's device and leaves the caller's current device as it found it (a process may
 // drive plans on several GPUs, and torch allocates on the current device).
@@ -103,41 +97,13 @@ void dev_free(void *ptr) {
     if (device_pool()) cudaFreeAsync(ptr, 0); else cudaFree(ptr);
 }
 
-template <class T>
-int upload(T **dptr, const std::vector<T> &v) {
-    *dptr = nullptr;
-    if (v.empty()) return AME_OK;
-    cudaError_t e = dev_alloc((void **)dptr, v.size() * sizeof(T));
-    if (e != cudaSuccess) return fail(AME_E_NOMEM, "device allocation of %zu bytes failed: %s", v.size() * sizeof(T), cudaGetErrorString(e));
-    CU(cudaMemcpy(*dptr, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return AME_OK;
-}
-
-constexpr int kLimMaxTile = 1 << 20;     // longest limiter tile (look-ahead + release of the slowest setting must fit one)
+constexpr int kEqBlock = 256;            // k_eq: 8 warps in ONE CTA per SM (two 4-warp CTAs were slower, see build_layout)
 constexpr int kMaxTimedSteps = 8;
 constexpr int kMaxTimedWaves = 128;
 constexpr int kTimedSlots = kMaxTimedWaves * AME_N_KERNELS;   // per step
 const char *const kKernelNames[AME_N_KERNELS] = {"k_eq", "k_band_split", "k_window_flag", "k_att_chain",
     "k_compress_apply", "k_kweight_energy", "k_tail_peak", "k_block_hist", "k_finalize", "k_apply_gain", "k_limiter", "k_true_peak"};
 enum { S_EQ = 0, S_SPLIT, S_FLAG, S_CHAIN, S_APPLY, S_KW, S_TAIL, S_HIST, S_FIN, S_GAIN, S_LIM, S_TP };
-
-// A wave = a contiguous range of tracks whose jobs are contiguous in every job table.  The device path
-// launches each kernel ONCE over all waves; the host path (ame_master_host) launches wave by wave so the
-// H2D copy of wave w+1 and the D2H copy of wave w-1 overlap the kernels of wave w.
-struct Wave {
-    int track_lo = 0, track_hi = 0;
-    int64_t frame_lo = 0, frame_hi = 0;            // packed-buffer range (multiples of 8 frames)
-    int eq_lo = 0, eq_n = 0, split_lo = 0, split_n = 0, chain_lo = 0, chain_n = 0, wf_lo = 0, wf_n = 0;
-    int chunk_lo = 0, chunk_n = 0, kw_lo = 0, kw_n = 0, gain_lo = 0, gain_n = 0, lim_lo = 0, lim_n = 0;
-    int64_t seg_lo = 0, seg_hi = 0;
-    int slot = 0;                                  // workspace slot (and stream) this wave runs in
-    bool limiter = false;                          // a track of the wave has the limiter stage
-    bool true_peak = false;                        // a track of the wave wants its oversampled peak
-    int64_t mb_frames = 0, n_groups = 0;           // of the wave's own multiband packing
-    bool xover_uni = false, kw_uni = false;        // all multiband tracks share the crossover / all k_kweight_energy tracks the K filter
-    XoverCfg xover{};
-    KwCfg kw{};
-};
 
 // Per-wave workspace.  A plan has n_slots of them; wave w runs in slot w % n_slots on that slot's stream, so a slot is
 // recycled in stream order and a plan over many waves needs the intermediate buffers of only n_slots waves.
@@ -159,22 +125,13 @@ struct Slot {
 
 }  // namespace
 
-struct ame_plan {
+// A plan is its layout (ame_layout.h) plus the device state built from it.
+struct ame_plan : Layout {
     int device = 0;
     int n_tracks = 0;
-    std::vector<ame_track_params> tracks;
-    std::vector<int64_t> mb_offset;       // per track, -1 if not multiband
-    std::vector<TrackDev> tdev;
-    std::vector<Wave> waves;
-    Wave all;                             // the union of all waves
-    int64_t total_frames = 0;             // padded
-    int64_t mb_frames = 0;                // padded; the largest wave's multiband packing = plane stride of every slot
-    int64_t slot_frames = 0, slot_groups = 0;
-    int slot_tiles = 0, slot_chains = 0;
-    int64_t n_sb_total = 0;
-    int eq_tile = 0, split_tile = 0, kw_tile_sb = 0;
     int n_sm = 148, chain_warps = 0;      // see chain_lanes()
     int precision = 0;                    // 1 = the FP32 EQ experiment
+    std::vector<void *> allocs;           // every device allocation of the plan (plan_alloc), freed by ame_plan_destroy
     size_t ws_bytes = 0;
     int64_t launches = 0;
     // device
@@ -186,7 +143,7 @@ struct ame_plan {
     WfJob *d_wf_jobs = nullptr;
     MbChunk *d_mb_chunks = nullptr;
     KwJob *d_kw_jobs = nullptr;
-    GainJob *d_gain_jobs = nullptr, *d_lim_jobs = nullptr;   // limiter tiles: the same (begin, end, track) records, shorter tiles
+    GainJob *d_gain_jobs = nullptr, *d_lim_jobs = nullptr;
     AttEntry *d_tables = nullptr;
     double *d_luts = nullptr;
     int n_luts = 0;
@@ -198,10 +155,7 @@ struct ame_plan {
     int *d_hist_st = nullptr;               // short-term (3 s) histogram per track, for loudness range
     int *d_peak = nullptr;
     unsigned *d_tp = nullptr;               // per track: float bits of the oversampled peak (k_true_peak)
-    bool any_limiter = false, any_tp = false;
-    int lim_keep = 2;                       // queue entries a recorded limiter state holds: look-ahead frames + 2
     int *d_lim_stats = nullptr;             // open tiles after the limiter's round 0 / 1 / 2, accumulated
-    int slot_lim_jobs = 0;
     ame_track_result *d_results = nullptr;
     cudaStream_t s_in = nullptr, s_out = nullptr;                       // host path: copy-in / copy-out
     std::vector<cudaEvent_t> ev_in, ev_run;                             // per wave
@@ -232,192 +186,31 @@ inline void t_end(ame_plan *p, int kernel, cudaStream_t s) {
     }
 }
 
-int dmalloc(ame_plan *p, void **ptr, size_t bytes) {
+// The one allocator of a plan's device memory: it records every pointer, and ame_plan_destroy frees what it recorded.
+int plan_alloc(ame_plan *p, void **ptr, size_t bytes) {
     *ptr = nullptr;
     if (bytes == 0) return AME_OK;
     cudaError_t e = dev_alloc(ptr, bytes);
-    if (e != cudaSuccess) return fail(AME_E_NOMEM, "device allocation of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
-    p->ws_bytes += bytes;
+    if (e != cudaSuccess) {
+        *ptr = nullptr;
+        return fail(AME_E_NOMEM, "device allocation of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
+    }
+    p->allocs.push_back(*ptr);
     return AME_OK;
 }
 
-// split chunk [cb, ce) into ceil(n / T) near-equal tiles whose interior boundaries are multiples of 8
-void tile_jobs(std::vector<TileJob> &out, int track, int variant, int64_t cb, int64_t ce, int64_t T) {
-    const int64_t n = ce - cb;
-    if (n <= 0) return;
-    const int64_t k = (n + T - 1) / T;
-    const int64_t t = align_up((n + k - 1) / k, 8);
-    int64_t b = cb;
-    while (b < ce) {
-        int64_t e = (b + t) & ~(int64_t)7;
-        if (e <= b) e = b + t;
-        if (e > ce) e = ce;
-        out.push_back(TileJob{cb, b, e, track, variant});
-        b = e;
-    }
+// workspace: counted by ame_plan_workspace_bytes, which leaves the uploaded tables out
+int dmalloc(ame_plan *p, void **ptr, size_t bytes) {
+    const int rc = plan_alloc(p, ptr, bytes);
+    if (rc == AME_OK) p->ws_bytes += bytes;
+    return rc;
 }
 
-// smallest tile (multiple of 8, >= min_tile) whose job count fits `slots` threads
-int64_t pick_tile(const std::vector<int64_t> &chunks, int64_t slots, int64_t min_tile) {
-    auto count = [&](int64_t T) {
-        int64_t jobs = 0;
-        for (int64_t n : chunks) jobs += (n + T - 1) / T;
-        return jobs;
-    };
-    int64_t lo = min_tile, hi = min_tile;
-    for (int64_t n : chunks) hi = std::max(hi, align_up(n, 8));
-    if (count(lo) <= slots) return lo;
-    while (lo < hi) {                    // count() is non-increasing in T
-        const int64_t mid = align_up((lo + hi) / 2, 8);
-        if (mid >= hi) break;
-        if (count(mid) <= slots) hi = mid; else lo = mid + 8;
-    }
-    return hi;
-}
-
-// k_eq tiles are cost-balanced: a thread's work is about (tile + warm-up) * cost-per-frame, and the cost per
-// frame differs a lot between tracks (no EQ at all ... 4 stages + warmth).  Give every track the tile length
-// that makes (T + warm) * cost equal to one common budget, the smallest budget whose job count fits `slots`.
-double eq_cost_per_frame(const ame_track_params &t) {
-    // relative cost of one frame in each k_eq variant, fitted to launches of 96 identical tracks per variant
-    // (profiles/r02/eq_variant_cost.txt, warm-up overlap taken out): 4 stages = 128, 2 shelves + 1 peak = 91, one peak 57,
-    // two shelves 58, no EQ 47 (bound by its loads, not by arithmetic); warmth + 26 (+ 20 without EQ); width is free
-    double c = 24.0;                                    // unpack, convert, pack, store
-    if (t.eq[0].kind != AME_EQ_BYPASS) c += 16.0;       // one section + blend, two channels
-    if (t.eq[1].kind != AME_EQ_BYPASS) c += 36.0;       // four sections + blend, two channels
-    if (t.eq[2].kind != AME_EQ_BYPASS) c += 36.0;
-    if (t.eq[3].kind != AME_EQ_BYPASS) c += 16.0;
-    const bool warm = (t.flags & AME_F_WARMTH) != 0;
-    if (c == 24.0) return warm ? 67.0 : 47.0;
-    return c + (warm ? 26.0 : 0.0);                     // two table look-ups + the 2x2 mix in explicit FP64 ops
-}
-
-// k_eq runs one thread per tile and switches on the track's variant, so a warp that mixes VARIANTS would run
-// both one after the other; tracks of the same variant can share a warp (coefficients are per-thread registers).
-// Every track gets a number of jobs (threads) in proportion to its cost (frames x cost per frame); the jobs of a
-// wave are then laid out variant by variant and only the end of each variant's run is padded to a whole warp.
-// (Until late in round 2 every track got whole WARPS: with ~9 warps per track the rounding left the cheapest
-// tracks of a 128-track launch with 14 % more work per thread than the mean, and the launch ended with them.)
-int eq_variant_of(const ame_track_params &t) {
-    int variant = 0;
-    for (int s = 0; s < 4; ++s)
-        if (t.eq[s].kind != AME_EQ_BYPASS) variant |= 1 << s;
-    if (t.flags & AME_F_WARMTH) variant |= 16;
-    return variant;
-}
-
-inline int eq_block() {          // 8 warps in ONE CTA per SM (experiments: AME_EQ_BLOCK=128 = two 4-warp CTAs)
-    static const int b = [] { const char *e = std::getenv("AME_EQ_BLOCK"); return (e && std::atoi(e) == 128) ? 128 : 256; }();
-    return b;
-}
-
-// Threads handed out = the resident set minus the padding at the end of every variant's run (a warp).  Padding the runs to
-// whole 8-warp CTAs (no CTA would mix two variants) was measured too: 9.84 ms against 9.69 ms on the 128-track launch -
-// the ~4 % of idle threads cost more than the ~12 mixed CTAs.
-std::vector<int64_t> eq_jobs_per_track(const ame_track_params *tracks, const std::vector<std::vector<int64_t>> &chunks,
-                                       const std::vector<double> &cost, int t_lo, int t_hi, int64_t slots, int64_t min_tile) {
-    const int n = (int)chunks.size();
-    std::vector<int64_t> jobs(n, 0), cap(n, 0), floor_jobs(n, 0);
-    std::vector<double> weight(n, 0.0);
-    double wsum = 0;
-    unsigned variants = 0;
-    int n_variants = 0;
-    for (int t = t_lo; t < t_hi; ++t) {
-        int64_t frames = 0, max_jobs = 0;
-        for (int64_t c : chunks[t]) { frames += c; max_jobs += std::max<int64_t>(1, c / min_tile); }
-        weight[t] = (double)frames * cost[t];
-        cap[t] = std::max<int64_t>(1, max_jobs);
-        floor_jobs[t] = std::max<int64_t>(1, (int64_t)chunks[t].size());      // tile_jobs makes one job per chunk at least
-        wsum += weight[t];
-        const unsigned bit = 1u << eq_variant_of(tracks[t]);
-        if (!(variants & bit)) { variants |= bit; ++n_variants; }
-    }
-    const int64_t avail = std::max<int64_t>(32 * (int64_t)(t_hi - t_lo), slots) - 31 * (int64_t)n_variants;
-    std::vector<std::pair<double, int>> rem;
-    int64_t used = 0;
-    for (int t = t_lo; t < t_hi; ++t) {
-        const double share = wsum > 0 ? (double)avail * weight[t] / wsum : 32.0;
-        jobs[t] = std::min(cap[t], std::max(floor_jobs[t], (int64_t)share));
-        used += jobs[t];
-        rem.emplace_back(share - (double)jobs[t], t);
-    }
-    std::sort(rem.begin(), rem.end(), [](const std::pair<double, int> &a, const std::pair<double, int> &b) { return a.first > b.first; });
-    for (size_t i = 0; i < rem.size() && used < avail; ++i)
-        if (jobs[rem[i].second] < cap[rem[i].second]) { ++jobs[rem[i].second]; ++used; }
-    return jobs;
-}
-
-int validate(const ame_track_params &t, int idx) {
-    if (t.n_frames < 0 || t.offset_frames < 0 || (t.offset_frames & 7))
-        return fail(AME_E_INVALID, "track %d: offset_frames must be a non-negative multiple of 8", idx);
-    if (t.sample_rate < 8000 || t.sample_rate > 384000)
-        return fail(AME_E_INVALID, "track %d: unsupported sample rate %d", idx, t.sample_rate);
-    if (t.halo_frames < 0 || (t.halo_frames & 7) || t.halo_frames % ((t.sample_rate + 5) / 10))
-        return fail(AME_E_INVALID, "track %d: halo_frames must be a multiple of 8 and of the 100 ms sub-block", idx);
-    if (t.warm_eq < 0 || t.warm_xover < 0 || t.warm_kw < 0)
-        return fail(AME_E_INVALID, "track %d: negative warm-up", idx);
-    if (t.flags & AME_F_LIMITER) {
-        if (t.halo_frames)
-            return fail(AME_E_UNSUPPORTED, "track %d: the limiter is one sequential state machine over the whole track and cannot "
-                                           "run on a time shard; limit the gathered output instead", idx);
-        if (t.lim_frames < 1 || t.lim_frames > kLimQueue - 24 || !(t.lim_limit > 0.0 && t.lim_limit <= 1.0) || !(t.lim_fs_release > 0.0) ||
-            t.lim_release_frames < 1 || t.lim_frames + t.lim_release_frames + 8 > kLimMaxTile || t.lim_thr_i < 1)
-            return fail(AME_E_INVALID, "track %d: bad limiter parameters (look-ahead %d frames, release %d frames)", idx, t.lim_frames,
-                        t.lim_release_frames);
-    }
-    for (int s = 0; s < 4; ++s) {
-        const int k = t.eq[s].kind;
-        const bool shelf = (s == 0 || s == 3);
-        if (k == AME_EQ_BYPASS) continue;
-        if (shelf ? (k != AME_EQ_SHELF_BOOST && k != AME_EQ_SHELF_CUT) : (k != AME_EQ_PEAK))
-            return fail(AME_E_INVALID, "track %d: eq stage %d has kind %d", idx, s, k);
-    }
-    // the kernels rely on the Butterworth numerator shape b0 * (1 +- 2 z^-1 + z^-2) that scipy.signal.butter
-    // produces for every filter of the reference (sign pattern and unit-gain sections are fixed by design)
-    auto shape = [&](const ame_biquad &q, double sgn, bool unit) {
-        return q.b1 == sgn * 2.0 * q.b0 && q.b2 == q.b0 && (!unit || q.b0 == 1.0);
-    };
-    bool ok = true;
-    if (t.eq[0].kind != AME_EQ_BYPASS) ok = ok && shape(t.eq[0].s[0], 1, false);
-    if (t.eq[3].kind != AME_EQ_BYPASS) ok = ok && shape(t.eq[3].s[0], -1, false);
-    for (int s = 1; s <= 2; ++s)
-        if (t.eq[s].kind != AME_EQ_BYPASS)
-            ok = ok && shape(t.eq[s].s[0], 1, false) && shape(t.eq[s].s[1], 1, true) && shape(t.eq[s].s[2], -1, true) &&
-                 shape(t.eq[s].s[3], -1, true);
-    if (t.flags & AME_F_MULTIBAND)
-        ok = ok && shape(t.xlp[0], 1, false) && shape(t.xlp[1], 1, true) && shape(t.xhp[0], -1, false) && shape(t.xhp[1], -1, true);
-    if (!ok) return fail(AME_E_UNSUPPORTED, "track %d: a filter section is not of Butterworth shape b0*(1 +- 2z^-1 + z^-2)", idx);
-    if (t.flags & AME_F_MULTIBAND)
-        for (int b = 0; b < 3; ++b) {
-            const ame_comp_band &c = t.comp[b];
-            if (!(c.thresh_rms >= 0) || !(c.attack_frames > 0) || !(c.release_frames > 0) || c.look_frames < 0 ||
-                c.look_frames > 4096)
-                return fail(AME_E_INVALID, "track %d: bad compressor band %d", idx, b);
-        }
+template <class T>
+int upload(ame_plan *p, T **dptr, const std::vector<T> &v) {
+    if (int rc = plan_alloc(p, (void **)dptr, v.size() * sizeof(T))) return rc;
+    if (!v.empty()) CU(cudaMemcpy(*dptr, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
     return AME_OK;
-}
-
-// pydub: (1 - 1/ratio) * max(20 * math.log(rms / thresh_rms, 10), 0); CPython's two-argument log is
-// log(x) / log(base) on the platform libm.  tau: smallest a >= 0 with fl(a + inc) >= m.
-void build_att_table(AttEntry *e, const ame_comp_band &c) {
-    const double ln10 = std::log(10.0);
-    for (int r = 0; r <= 32768; ++r) {
-        double over = 0.0;
-        if (r != 0) {
-            const double ratio = (double)r / c.thresh_rms;
-            if (ratio != 0.0) {
-                const double db = 20 * (std::log(ratio) / ln10);
-                over = db > 0 ? db : 0.0;
-            }
-        }
-        const double m = c.coef * over;
-        const double inc = m / c.attack_frames;
-        double tau = m - inc;
-        if (!(tau > 0)) tau = 0.0;
-        while (tau > 0 && tau + inc >= m) tau = std::nextafter(tau, -1.0);
-        while (tau + inc < m) tau = std::nextafter(tau, 1e300);
-        e[r] = AttEntry{m, inc, m / c.release_frames, tau};
-    }
 }
 
 #define LAUNCH_CHECK(p)                                                                            \
@@ -467,25 +260,25 @@ Bufs slot_bufs(ame_plan *p, const Wave &w, const int16_t *d_in, int16_t *d_out) 
 }
 
 int run_eq(ame_plan *p, const Wave &w, const int16_t *d_in, int16_t *d_pre, cudaStream_t s) {
-    if (!w.eq_n) return AME_OK;
+    if (!w.eq.n) return AME_OK;
     t_begin(p, S_EQ, s);
     if (p->precision == 1)
-        k_eq_f32<<<(w.eq_n + 127) / 128, 128, 0, s>>>(p->d_eq_jobs + w.eq_lo, w.eq_n, p->d_tracks, p->d_luts, d_in, d_pre);
+        k_eq_f32<<<(w.eq.n + 127) / 128, 128, 0, s>>>(p->d_eq_jobs + w.eq.lo, w.eq.n, p->d_tracks, p->d_luts, d_in, d_pre);
     else
-        k_eq<<<(w.eq_n + eq_block() - 1) / eq_block(), eq_block(), 0, s>>>(p->d_eq_jobs + w.eq_lo, w.eq_n, p->d_tracks, p->d_luts, d_in, d_pre);
+        k_eq<<<(w.eq.n + kEqBlock - 1) / kEqBlock, kEqBlock, 0, s>>>(p->d_eq_jobs + w.eq.lo, w.eq.n, p->d_tracks, p->d_luts, d_in, d_pre);
     LAUNCH_CHECK(p);
     t_end(p, S_EQ, s);
     return AME_OK;
 }
 
 int run_split(ame_plan *p, const Wave &w, const int16_t *d_pre, int16_t *d_bands, cudaStream_t s) {
-    if (!w.split_n) return AME_OK;
+    if (!w.split.n) return AME_OK;
     t_begin(p, S_SPLIT, s);
     if (w.xover_uni)
-        k_band_split<true><<<(w.split_n + 127) / 128, 128, 0, s>>>(w.xover, p->d_split_jobs + w.split_lo, w.split_n, p->d_tracks, p->d_mb_delta,
+        k_band_split<true><<<(w.split.n + 127) / 128, 128, 0, s>>>(w.xover, p->d_split_jobs + w.split.lo, w.split.n, p->d_tracks, p->d_mb_delta,
                                                                    d_pre, d_bands, p->mb_frames);
     else
-        k_band_split<false><<<(w.split_n + 127) / 128, 128, 0, s>>>(w.xover, p->d_split_jobs + w.split_lo, w.split_n, p->d_tracks, p->d_mb_delta,
+        k_band_split<false><<<(w.split.n + 127) / 128, 128, 0, s>>>(w.xover, p->d_split_jobs + w.split.lo, w.split.n, p->d_tracks, p->d_mb_delta,
                                                                     d_pre, d_bands, p->mb_frames);
     LAUNCH_CHECK(p);
     t_end(p, S_SPLIT, s);
@@ -505,25 +298,25 @@ int chain_lanes(const ame_plan *p, int n_chains) {
 }
 
 int run_compress(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
-    if (!w.chain_n) return AME_OK;
+    if (!w.chain.n) return AME_OK;
     t_begin(p, S_FLAG, s);
     int *tile_base = b.tile_cnt + std::max(p->slot_tiles, 1);
-    k_window_flag<<<w.wf_n, kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf_lo, b.bands, b.rms, b.tile_cnt, b.grp);
+    k_window_flag<<<w.wf.n, kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf.lo, b.bands, b.rms, b.tile_cnt, b.grp);
     LAUNCH_CHECK(p);
-    k_tile_prefix<<<w.chain_n, kWfThreads, 0, s>>>(p->d_chain_jobs + w.chain_lo, b.tile_cnt, tile_base, b.n_flagged);
+    k_tile_prefix<<<w.chain.n, kWfThreads, 0, s>>>(p->d_chain_jobs + w.chain.lo, b.tile_cnt, tile_base, b.n_flagged);
     LAUNCH_CHECK(p);
-    k_compact<<<(w.wf_n + kWfThreads / 32 - 1) / (kWfThreads / 32), kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf_lo, w.wf_n, b.rms, b.tile_cnt,
+    k_compact<<<(w.wf.n + kWfThreads / 32 - 1) / (kWfThreads / 32), kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf.lo, w.wf.n, b.rms, b.tile_cnt,
                                                                                           tile_base, b.list, b.grp);
     LAUNCH_CHECK(p);
     t_end(p, S_FLAG, s);
     t_begin(p, S_CHAIN, s);
-    const int lanes = chain_lanes(p, w.chain_n);
-    k_att_chain<<<w.chain_n, std::max(lanes, 32), 0, s>>>(p->d_chain_jobs + w.chain_lo, b.list, b.n_flagged, p->d_tables, b.att, p->mb_frames,
-                                            lanes, p->d_chain_stats + 2 * (size_t)w.chain_lo);
+    const int lanes = chain_lanes(p, w.chain.n);
+    k_att_chain<<<w.chain.n, std::max(lanes, 32), 0, s>>>(p->d_chain_jobs + w.chain.lo, b.list, b.n_flagged, p->d_tables, b.att, p->mb_frames,
+                                            lanes, p->d_chain_stats + 2 * (size_t)w.chain.lo);
     LAUNCH_CHECK(p);
     t_end(p, S_CHAIN, s);
     t_begin(p, S_APPLY, s);
-    k_compress_apply<<<(unsigned)((w.seg_hi - w.seg_lo + 3) / 4), 128, 0, s>>>(p->d_mb_chunks + w.chunk_lo, w.chunk_n, w.seg_lo, w.seg_hi,
+    k_compress_apply<<<(unsigned)((w.seg_hi - w.seg_lo + 3) / 4), 128, 0, s>>>(p->d_mb_chunks + w.mb_chunks.lo, w.mb_chunks.n, w.seg_lo, w.seg_hi,
                                                                                 b.bands, b.grp, b.att, b.pre, p->mb_frames);
     LAUNCH_CHECK(p);
     t_end(p, S_APPLY, s);
@@ -534,13 +327,13 @@ int run_hist(ame_plan *p, const Wave &w, const int16_t *d_pre, int64_t *d_hist, 
     const int nt = w.track_hi - w.track_lo;
     if (nt <= 0) return AME_OK;
     CU(cudaMemsetAsync(p->d_peak + w.track_lo, 0, (size_t)nt * 4, s));
-    if (w.kw_n) {
+    if (w.kw.n) {
         t_begin(p, S_KW, s);
         if (w.kw_uni)
-            k_kweight_energy<true><<<(w.kw_n + 127) / 128, 128, 0, s>>>(w.kw, p->d_kw_jobs + w.kw_lo, w.kw_n, p->d_tracks, p->d_tdev, d_pre,
+            k_kweight_energy<true><<<(w.kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_kw_jobs + w.kw.lo, w.kw.n, p->d_tracks, p->d_tdev, d_pre,
                                                                         p->d_energy, p->d_peak);
         else
-            k_kweight_energy<false><<<(w.kw_n + 127) / 128, 128, 0, s>>>(w.kw, p->d_kw_jobs + w.kw_lo, w.kw_n, p->d_tracks, p->d_tdev, d_pre,
+            k_kweight_energy<false><<<(w.kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_kw_jobs + w.kw.lo, w.kw.n, p->d_tracks, p->d_tdev, d_pre,
                                                                          p->d_energy, p->d_peak);
         LAUNCH_CHECK(p);
         t_end(p, S_KW, s);
@@ -550,9 +343,9 @@ int run_hist(ame_plan *p, const Wave &w, const int16_t *d_pre, int64_t *d_hist, 
     LAUNCH_CHECK(p);
     t_end(p, S_TAIL, s);
     CU(cudaMemsetAsync(p->d_tp + w.track_lo, 0, (size_t)nt * 4, s));
-    if (w.true_peak && w.gain_n) {
+    if (w.true_peak && w.gain.n) {
         t_begin(p, S_TP, s);
-        k_true_peak<<<w.gain_n, 256, 0, s>>>(p->d_gain_jobs + w.gain_lo, p->d_tracks, d_pre, p->d_tp);
+        k_true_peak<<<w.gain.n, 256, 0, s>>>(p->d_gain_jobs + w.gain.lo, p->d_tracks, d_pre, p->d_tp);
         LAUNCH_CHECK(p);
         t_end(p, S_TP, s);
     }
@@ -567,31 +360,31 @@ int run_hist(ame_plan *p, const Wave &w, const int16_t *d_pre, int64_t *d_hist, 
 int run_apply(ame_plan *p, const Wave &w, const int16_t *d_pre, int16_t *d_out, const Bufs &b, cudaStream_t s) {
     int16_t *d_norm = b.norm;
     long long *lim_last = b.lim_last;
-    if (!w.gain_n) return AME_OK;
+    if (!w.gain.n) return AME_OK;
     t_begin(p, S_GAIN, s);
-    if (w.limiter) CU(cudaMemsetAsync(lim_last, 0xff, (size_t)w.lim_n * sizeof(long long), s));      // -1: no frame over the limit
-    k_apply_gain<<<w.gain_n, 256, 0, s>>>(p->d_gain_jobs + w.gain_lo, p->d_results, p->d_tracks, p->d_tdev, d_pre, d_out, d_norm, lim_last);
+    if (w.limiter) CU(cudaMemsetAsync(lim_last, 0xff, (size_t)w.lim.n * sizeof(long long), s));      // -1: no frame over the limit
+    k_apply_gain<<<w.gain.n, 256, 0, s>>>(p->d_gain_jobs + w.gain.lo, p->d_results, p->d_tracks, p->d_tdev, d_pre, d_out, d_norm, lim_last);
     LAUNCH_CHECK(p);
     t_end(p, S_GAIN, s);
     if (w.limiter) {
         t_begin(p, S_LIM, s);
-        const GainJob *gj = p->d_lim_jobs + w.lim_lo;
+        const GainJob *gj = p->d_lim_jobs + w.lim.lo;
         constexpr int kLimRounds = 2;                 // repair rounds before the sequential fallback
         int cap = 64;
         while (cap < p->lim_keep + 2) cap *= 2;       // queue capacity in shared memory: a power of two
         const size_t smem = lim_smem_bytes(cap);
         for (int round = 0; round <= kLimRounds; ++round) {
             if (round == 0) {                         // the elementwise tiles, 256 threads each
-                k_limiter<<<w.lim_n, 256, smem, s>>>(gj, w.lim_n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, 0, cap);
+                k_limiter<<<w.lim.n, 256, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, 0, cap);
                 LAUNCH_CHECK(p);
             }
-            k_limiter<<<w.lim_n, 32, smem, s>>>(gj, w.lim_n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, round, cap);
+            k_limiter<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, round, cap);
             LAUNCH_CHECK(p);
-            k_lim_verify<<<(w.lim_n + 3) / 4, 128, 0, s>>>(gj, w.lim_n, p->d_tracks, b.lim_in, b.lim_out, b.lim_need,
+            k_lim_verify<<<(w.lim.n + 3) / 4, 128, 0, s>>>(gj, w.lim.n, p->d_tracks, b.lim_in, b.lim_out, b.lim_need,
                                                              p->d_lim_stats + round);
             LAUNCH_CHECK(p);
         }
-        k_lim_fallback<<<w.lim_n, 32, smem, s>>>(gj, w.lim_n, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, cap);
+        k_lim_fallback<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, cap);
         LAUNCH_CHECK(p);
         t_end(p, S_LIM, s);
     }
@@ -651,20 +444,10 @@ int ame_device_count(int *count) {
 void ame_plan_destroy(ame_plan *p) {
     if (!p) return;
     DeviceGuard guard(p->device);
-    void *ptrs[] = {p->d_tracks, p->d_tdev, p->d_mb_delta, p->d_eq_jobs, p->d_split_jobs, p->d_wf_jobs, p->d_mb_chunks,
-                    p->d_chain_jobs, p->d_kw_jobs, p->d_gain_jobs, p->d_lim_jobs, p->d_tables, p->d_luts,
-                    p->d_in, p->d_out, p->d_energy, p->d_hist, p->d_hist_st, p->d_peak, p->d_tp, p->d_lim_stats, p->d_results,
-                    p->d_chain_stats};
     cudaDeviceSynchronize();            // nothing of this plan may still be running when its memory goes back to the pool
-    for (void *q : ptrs) dev_free(q);
-    for (Slot &sl : p->slots) {
-        for (void *q : {(void *)sl.pre, (void *)sl.bands, (void *)sl.rms, (void *)sl.list, (void *)sl.tile_cnt, (void *)sl.n_flagged,
-                        (void *)sl.grp, (void *)sl.att, (void *)sl.norm, (void *)sl.lim_last, (void *)sl.lim_in.st, (void *)sl.lim_in.qframe,
-                        (void *)sl.lim_in.qdelta, (void *)sl.lim_out.st, (void *)sl.lim_out.qframe, (void *)sl.lim_out.qdelta,
-                        (void *)sl.lim_need})
-            dev_free(q);
+    for (void *q : p->allocs) dev_free(q);
+    for (Slot &sl : p->slots)
         if (sl.stream) cudaStreamDestroy(sl.stream);
-    }
     for (cudaStream_t s : {p->s_in, p->s_out})
         if (s) cudaStreamDestroy(s);
     for (cudaEvent_t e : p->ev_in) cudaEventDestroy(e);
@@ -689,340 +472,34 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
     ame_plan *p = new ame_plan();
     p->device = device;
     p->n_tracks = n_tracks;
-    p->tracks.assign(tracks, tracks + n_tracks);
-    int rc = AME_OK;
-    auto bail = [&](int code) { ame_plan_destroy(p); return code; };
-
-    // ---- layout -------------------------------------------------------------------------------
-    std::vector<std::pair<int64_t, int64_t>> spans;
-    p->mb_offset.assign(n_tracks, -1);
-    p->tdev.resize(n_tracks);
-    int64_t sum_frames = 0;
-    for (int t = 0; t < n_tracks; ++t) {
-        ame_track_params &tp = p->tracks[t];
-        if ((rc = validate(tp, t)) != AME_OK) return bail(rc);
-        const int64_t n_total = tp.halo_frames + tp.n_frames;
-        if (t && tp.offset_frames < p->tracks[t - 1].offset_frames)
-            return bail(fail(AME_E_INVALID, "tracks must be ordered by offset_frames"));
-        spans.emplace_back(tp.offset_frames, tp.offset_frames + n_total);
-        p->total_frames = std::max(p->total_frames, align_up(tp.offset_frames + n_total, 8));
-        sum_frames += tp.n_frames;
-        const int s100 = (tp.sample_rate + 5) / 10;
-        p->tdev[t].s100 = s100;
-        p->tdev[t].n_sb = (int)(n_total / s100);
-        p->tdev[t].n_total = n_total;
-        // blocks whose last sub-block lies in the halo were counted by the previous shard
-        p->tdev[t].first_block = tp.halo_frames ? std::max<int>(0, (int)(tp.halo_frames / s100) - 3) : 0;
-        p->tdev[t].sb_offset = p->n_sb_total;
-        p->n_sb_total += p->tdev[t].n_sb;
-        p->tdev[t].pad = 0;
-        p->tdev[t].lim_tile0 = 0;
-        p->tdev[t].lim_shift = 15;
-        p->any_limiter = p->any_limiter || (tp.flags & AME_F_LIMITER);
-        if (tp.flags & AME_F_LIMITER) p->lim_keep = std::max(p->lim_keep, tp.lim_frames + 2);
-        p->any_tp = p->any_tp || (tp.flags & AME_F_TRUE_PEAK);
-    }
-    for (size_t i = 1; i < spans.size(); ++i)
-        if (spans[i].first < align_up(spans[i - 1].second, 8)) return bail(fail(AME_E_INVALID, "tracks overlap in the packed buffer"));
-    if (p->total_frames == 0) p->total_frames = 8;
-
-    // ---- waves: contiguous track ranges with about equal frames ----------------------------------
-    int n_waves = o.n_waves > 0 ? o.n_waves : 1;
-    n_waves = std::max(1, std::min(n_waves, n_tracks));
-    {
-        // With many waves the FIRST wave is a single track: in the host path nothing can be copied back before the
-        // first wave has been copied in and mastered, so a small first wave starts the D2H stream early.
-        p->waves.resize(n_waves);
-        const bool small_first = o.host_io && n_waves >= 4 && n_tracks >= 2 * n_waves;
-        int t = 0;
-        int64_t acc = 0;
-        const int64_t first_frames = small_first ? p->tracks[0].n_frames : 0;
-        for (int w = 0; w < n_waves; ++w) {
-            Wave &wv = p->waves[w];
-            wv.track_lo = t;
-            const int must_leave = n_waves - 1 - w;                 // at least one track for every later wave
-            if (small_first && w == 0) {
-                acc += p->tracks[t++].n_frames;
-            } else {
-                const int64_t share = small_first ? w : w + 1;
-                const int64_t parts = small_first ? n_waves - 1 : n_waves;
-                const int64_t target = first_frames + (sum_frames - first_frames) * share / parts;
-                while (t < n_tracks - must_leave && (t == wv.track_lo || acc + p->tracks[t].n_frames / 2 <= target)) acc += p->tracks[t++].n_frames;
-            }
-            if (w == n_waves - 1) t = n_tracks;
-            wv.track_hi = t;
-            wv.frame_lo = p->tracks[wv.track_lo].offset_frames;
-            wv.frame_hi = (wv.track_hi < n_tracks) ? p->tracks[wv.track_hi].offset_frames : p->total_frames;
-        }
-    }
-    // Slots: a wave's intermediate buffers (pre-normalisation signal, bands, rms, attenuations) live in slot
-    // w % n_slots and are recycled in stream order, so a batch far larger than the workspace can be planned.
-    int n_slots = o.n_slots > 0 ? o.n_slots : std::min(n_waves, 4);
-    n_slots = std::max(1, std::min(n_slots, n_waves));
-    for (int w = 0; w < n_waves; ++w) {
-        Wave &wv = p->waves[w];
-        wv.slot = w % n_slots;
-        int64_t mb = 0;
-        for (int t = wv.track_lo; t < wv.track_hi; ++t)
-            if (p->tracks[t].flags & AME_F_MULTIBAND) {
-                p->mb_offset[t] = mb;                               // within the wave's own multiband packing
-                mb += align_up(p->tdev[t].n_total, 8);
-            }
-        wv.mb_frames = mb;
-        p->mb_frames = std::max(p->mb_frames, mb);
-        p->slot_frames = std::max(p->slot_frames, wv.frame_hi - wv.frame_lo);
-    }
-
-    // ---- chunk geometry, tile sizes -----------------------------------------------------------------
-    // Tiles are sized so that ONE launch fills its share of the machine with one wave of resident threads (no tail
-    // wave).  Waves in different slots run concurrently, so a launch gets 1 / min(n_slots, 4) of the resident threads.
-    std::vector<std::vector<int64_t>> chunks_all(n_tracks);
-    for (int t = 0; t < n_tracks; ++t) {
-        const ame_track_params &tp = p->tracks[t];
-        const int64_t cf = tp.chunk_frames > 0 ? tp.chunk_frames : std::max<int64_t>(tp.n_frames, 1);
-        for (int64_t c0 = 0; c0 < tp.n_frames; c0 += cf) chunks_all[t].push_back(std::min(cf, tp.n_frames - c0));
-    }
-    int n_sm = 148, occ_eq = 2, occ_split = 3;
-    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
-    p->n_sm = n_sm;
     p->chain_warps = std::max(-1, std::min(o.chain_warps, kChainMaxThreads / 32));
     p->precision = o.precision == 1 ? 1 : 0;
-    if (p->precision == 1) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_eq, k_eq_f32, 128, 0);
-    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_eq, k_eq, 128, 0);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_split, k_band_split<true>, 128, 0);
-    if (const char *e = std::getenv("AME_EQ_CTAS_PER_SM")) occ_eq = std::max(1, std::atoi(e));       // experiments
-    if (const char *e = std::getenv("AME_SPLIT_CTAS_PER_SM")) occ_split = std::max(1, std::atoi(e));
-    const int share = std::min(n_slots, 4);
-    const int64_t eq_slots = (int64_t)n_sm * std::max(occ_eq, 1) * 128 / share;         // one thread per tile
-    const int64_t split_slots = (int64_t)n_sm * std::max(occ_split, 1) * 128 / share;
-    constexpr int64_t kMinTile = 512;
-    int64_t split_tile = kMinTile;
-    std::vector<double> eq_cost(n_tracks);
-    std::vector<int64_t> eq_want(n_tracks, 32);
-    int max_warm_kw = 0, min_s100 = 1 << 30;
-    for (int t = 0; t < n_tracks; ++t) {
-        eq_cost[t] = eq_cost_per_frame(p->tracks[t]);
-        max_warm_kw = std::max(max_warm_kw, p->tracks[t].warm_kw);
-        min_s100 = std::min(min_s100, p->tdev[t].s100);
-    }
-    const int64_t n_sb_kw = p->n_sb_total;
-    // One warp per scheduler already gives these FP64-bound kernels ~77 % of the throughput of two (k_eq alone: 13.7 vs
-    // 10.6 ms), and every tile pays its warm-up once: when a wave is so small that a full set of resident threads would
-    // make the tiles shorter than ~1.2 x the warm-up (one long 192 kHz track), half the threads do the job sooner -
-    // (2T + W) / (2T * 0.77) < (T + W) / T  <=>  T < 1.17 W.
-    auto fewer_threads = [](int64_t slots, double frames, double warm_weighted) {
-        const double tile = frames / (double)slots, warm = frames > 0 ? warm_weighted / frames : 0.0;
-        if (std::getenv("AME_FULL_THREADS")) return slots;      // experiments
-        return (tile < 1.17 * warm && slots >= 512) ? slots / 2 : slots;
-    };
-    for (const Wave &wv : p->waves) {
-        std::vector<int64_t> cm;
-        double eq_frames = 0, eq_warm = 0, mb_fr = 0, mb_warm = 0;
-        for (int t = wv.track_lo; t < wv.track_hi; ++t) {
-            const ame_track_params &tp = p->tracks[t];
-            eq_frames += (double)tp.n_frames;
-            eq_warm += (double)tp.n_frames * tp.warm_eq;
-            if (tp.flags & AME_F_MULTIBAND) {
-                cm.insert(cm.end(), chunks_all[t].begin(), chunks_all[t].end());
-                mb_fr += (double)tp.n_frames;
-                mb_warm += (double)tp.n_frames * tp.warm_xover;
-            }
-        }
-        split_tile = std::max(split_tile, pick_tile(cm, fewer_threads(split_slots, mb_fr, mb_warm), kMinTile));
-        const std::vector<int64_t> tw = eq_jobs_per_track(p->tracks.data(), chunks_all, eq_cost, wv.track_lo, wv.track_hi,
-                                                          fewer_threads(eq_slots, eq_frames, eq_warm), kMinTile);
-        for (int t = wv.track_lo; t < wv.track_hi; ++t) eq_want[t] = tw[t];
-    }
-    p->eq_tile = 0;
-    p->split_tile = o.xover_tile_frames > 0 ? (int)align_up(o.xover_tile_frames, 8) : (int)split_tile;
-    if (o.kw_tile_subblocks > 0) {
-        p->kw_tile_sb = o.kw_tile_subblocks;
-    } else if (n_sb_kw > 0) {
-        // a tile of sub-blocks costs (tile + warm-up) frames: keep the warm-up below ~15 % when the batch is big
-        // enough to still give every SM ~512 threads per launch, else shrink the tile towards one sub-block
-        const int64_t want = std::max<int64_t>(1, ((int64_t)max_warm_kw * 6 + min_s100 - 1) / min_s100);
-        const int64_t fill = std::max<int64_t>(1, n_sb_kw / n_waves * share / ((int64_t)n_sm * 512));
-        p->kw_tile_sb = (int)std::min(want, fill);
-    } else {
-        p->kw_tile_sb = 1;
-    }
+    auto bail = [&](int code) { ame_plan_destroy(p); return code; };
 
-    // ---- job tables (every table is ordered by track, hence contiguous per wave) ---------------------
-    std::vector<TileJob> eq_jobs, split_jobs;
-    std::vector<ChainJob> chain_jobs;
-    std::vector<WfJob> wf_jobs;
-    std::vector<MbChunk> mb_chunks;
-    std::vector<KwJob> kw_jobs;
-    std::vector<GainJob> gain_jobs, lim_jobs;
-    std::vector<int64_t> mb_delta(n_tracks, 0);
-    std::vector<AttEntry> tables;
-    std::map<std::tuple<double, double, double, double>, int> table_index;
-    int64_t n_seg_total = 0;
-
-    for (Wave &wv : p->waves) {
-        wv.eq_lo = (int)eq_jobs.size(); wv.split_lo = (int)split_jobs.size(); wv.chain_lo = (int)chain_jobs.size();
-        wv.chunk_lo = (int)mb_chunks.size(); wv.kw_lo = (int)kw_jobs.size(); wv.gain_lo = (int)gain_jobs.size();
-        wv.lim_lo = (int)lim_jobs.size();
-        wv.seg_lo = n_seg_total;
-        int64_t n_groups = 0;                          // group records of this wave (slot-local indices)
-        std::map<int, std::vector<TileJob>> eq_bucket;   // k_eq jobs of this wave by variant (a warp runs ONE variant)
-        for (int t = wv.track_lo; t < wv.track_hi; ++t) {
-            ame_track_params &tp = p->tracks[t];
-            const int variant = eq_variant_of(tp);
-            const bool mb = (tp.flags & AME_F_MULTIBAND) != 0;
-            if (mb) {
-                mb_delta[t] = p->mb_offset[t] - tp.offset_frames;
-                for (int b = 0; b < 3; ++b) {
-                    ame_comp_band &c = tp.comp[b];
-                    auto key = std::make_tuple(c.thresh_rms, c.coef, c.attack_frames, c.release_frames);
-                    auto it = table_index.find(key);
-                    if (it == table_index.end()) {
-                        const int idx = (int)table_index.size();
-                        table_index[key] = idx;
-                        tables.resize(tables.size() + 32769);
-                        build_att_table(tables.data() + (size_t)idx * 32769, c);
-                        c.table = idx;
-                    } else {
-                        c.table = it->second;
-                    }
-                }
-            }
-            // k_eq jobs of this track: eq_want[t] jobs spread over the chunks by length (or the requested tile), collected
-            // per variant and laid out at the end of the wave
-            {
-                std::vector<TileJob> &bucket = eq_bucket[variant];
-                int64_t c0e = 0, jobs_before = 0;
-                int64_t nf = 0;
-                for (int64_t cn : chunks_all[t]) nf += cn;
-                nf = std::max<int64_t>(nf, 1);
-                const int64_t want = eq_want[t];
-                for (int64_t cn : chunks_all[t]) {
-                    const int64_t cb = tp.offset_frames + tp.halo_frames + c0e, ce = cb + cn;
-                    int64_t T;
-                    if (o.eq_tile_frames > 0) {
-                        T = align_up(o.eq_tile_frames, 8);
-                    } else {
-                        // cumulative rounding: the chunks together get exactly `want` jobs (never more)
-                        const int64_t upto = (int64_t)((__int128)want * (c0e + cn) / nf);
-                        const int64_t jc = std::max<int64_t>(1, upto - jobs_before);
-                        jobs_before = upto;
-                        T = std::max<int64_t>(kMinTile, align_up((cn + jc - 1) / jc, 8));
-                    }
-                    tile_jobs(bucket, t, variant, cb, ce, T);
-                    p->eq_tile = std::max<int>(p->eq_tile, (int)std::min<int64_t>(T, INT32_MAX));
-                    c0e += cn;
-                }
-            }
-            int64_t c0 = 0;
-            for (int64_t cn : chunks_all[t]) {
-                const int64_t cb = tp.offset_frames + tp.halo_frames + c0, ce = cb + cn;
-                if (mb) {
-                    tile_jobs(split_jobs, t, 0, cb, ce, p->split_tile);
-                    MbChunk ck{cb, p->mb_offset[t] + tp.halo_frames + c0, cn, n_seg_total, {0, 0, 0}, t, 0};
-                    for (int b = 0; b < 3; ++b) {
-                        const double thr = tp.comp[b].thresh_rms;
-                        const uint32_t thr_i = thr >= 65535.0 ? 0x7fffffffu : (uint32_t)std::floor(thr) + 1u;
-                        ck.grp_begin[b] = n_groups;
-                        chain_jobs.push_back(ChainJob{ck.mb_begin, cn, n_groups, b, tp.comp[b].table, thr_i, tp.comp[b].look_frames, 0, 0});
-                        n_groups += (cn + 31) / 32;
-                    }
-                    n_seg_total += (cn + kSeg - 1) / kSeg;
-                    mb_chunks.push_back(ck);
-                }
-                c0 += cn;
-            }
-            for (int sb = 0; sb < p->tdev[t].n_sb; sb += p->kw_tile_sb)
-                kw_jobs.push_back(KwJob{t, sb, std::min(sb + p->kw_tile_sb, p->tdev[t].n_sb), 0});
-            for (int64_t b = 0; b < tp.n_frames; b += kGainTile)
-                gain_jobs.push_back(GainJob{tp.offset_frames + tp.halo_frames + b,
-                                            tp.offset_frames + tp.halo_frames + std::min<int64_t>(b + kGainTile, tp.n_frames), t, 0});
-            if (tp.flags & AME_F_LIMITER) {
-                // limiter tiles: a power of two >= G = look-ahead + release + 8 (a tile without an over-limit frame then
-                // guarantees the initial state at its end), as short as that allows: more tiles = more warps in flight
-                const int64_t G = (int64_t)tp.lim_frames + tp.lim_release_frames + 8;
-                int shift = 13;
-                while ((1LL << shift) < G) ++shift;
-                p->tdev[t].lim_shift = shift;
-                p->tdev[t].lim_tile0 = (int)lim_jobs.size() - wv.lim_lo;
-                for (int64_t b = 0; b < tp.n_frames; b += 1LL << shift)
-                    lim_jobs.push_back(GainJob{tp.offset_frames + tp.halo_frames + b,
-                                               tp.offset_frames + tp.halo_frames + std::min<int64_t>(b + (1LL << shift), tp.n_frames), t, 0});
-            }
-        }
-        {
-            bool have_x = false, have_k = false;
-            wv.xover_uni = wv.kw_uni = true;
-            for (int t = wv.track_lo; t < wv.track_hi; ++t) {
-                const ame_track_params &tp = p->tracks[t];
-                if (tp.flags & AME_F_MULTIBAND) {
-                    const XoverCfg x{tp.xlp[0].b0, tp.xlp[0].a1, tp.xlp[0].a2, tp.xlp[1].a1, tp.xlp[1].a2,
-                                     tp.xhp[0].b0, tp.xhp[0].a1, tp.xhp[0].a2, tp.xhp[1].a1, tp.xhp[1].a2};
-                    if (!have_x) { wv.xover = x; have_x = true; }
-                    else if (std::memcmp(&x, &wv.xover, sizeof x)) wv.xover_uni = false;
-                }
-                {
-                    const KwCfg k{tp.kw[0].b0, tp.kw[0].b1, tp.kw[0].b2, tp.kw[0].a1, tp.kw[0].a2, tp.kw[1].a1, tp.kw[1].a2};
-                    const bool rlb = tp.kw[1].b0 == 1.0 && tp.kw[1].b1 == -2.0 && tp.kw[1].b2 == 1.0;
-                    if (!have_k) { wv.kw = k; have_k = true; }
-                    else if (std::memcmp(&k, &wv.kw, sizeof k)) wv.kw_uni = false;
-                    if (!rlb) wv.kw_uni = false;
-                }
-            }
-        }
-        wv.n_groups = n_groups;
-        p->slot_groups = std::max(p->slot_groups, n_groups);
-        // longest chains first inside the wave: the launch ends with its slowest CTA
-        std::stable_sort(chain_jobs.begin() + wv.chain_lo, chain_jobs.end(), [](const ChainJob &a, const ChainJob &b) { return a.n > b.n; });
-        wv.wf_lo = (int)wf_jobs.size();
-        for (int c = wv.chain_lo; c < (int)chain_jobs.size(); ++c) {
-            chain_jobs[c].tile0 = (int)wf_jobs.size() - wv.wf_lo;
-            const ChainJob &cj = chain_jobs[c];
-            for (int64_t tb = 0; tb < cj.n; tb += kWfTile)
-                wf_jobs.push_back(WfJob{tb, (int64_t)cj.band * p->mb_frames + cj.mb_begin, cj.n, cj.grp_begin, c, cj.look, cj.thr_i, cj.tile0});
-        }
-        {   // every variant's run is padded to whole warps (a warp runs ONE variant) and the runs follow one another; with one
-            // 8-warp CTA per SM nearly every SM then executes ONE variant - each variant is its own ~19 KB unrolled loop in
-            // the instruction cache (two 4-warp CTAs of different variants per SM: 10.5 ms on the 128-track launch, one 8-warp
-            // CTA: 9.7 ms).  Interleaving the variants' warps in proportion (every SM gets the wave's mix of FP64-heavy and
-            // load-bound warps; AME_EQ_INTERLEAVE) gave 18.0 ms: four loops per CTA (profiles/r02/summary.md).
-            std::vector<std::pair<double, std::pair<int, int>>> order;     // (position in [0, 1), (variant, warp of the variant))
-            for (auto &kv : eq_bucket) {
-                std::vector<TileJob> &b = kv.second;
-                if (b.empty()) continue;
-                TileJob d = b.back();
-                d.tile_begin = d.tile_end;
-                while (b.size() % 32) b.push_back(d);
-                const int nw = (int)(b.size() / 32);
-                for (int w = 0; w < nw; ++w) order.push_back({(w + 0.5) / nw, {kv.first, w}});
-            }
-            if (std::getenv("AME_EQ_INTERLEAVE")) std::stable_sort(order.begin(), order.end());   // experiment (see above): lost
-            for (const auto &o2 : order) {
-                const std::vector<TileJob> &b = eq_bucket[o2.second.first];
-                eq_jobs.insert(eq_jobs.end(), b.begin() + (size_t)o2.second.second * 32, b.begin() + (size_t)o2.second.second * 32 + 32);
-            }
-        }
-        wv.eq_n = (int)eq_jobs.size() - wv.eq_lo; wv.split_n = (int)split_jobs.size() - wv.split_lo;
-        wv.chain_n = (int)chain_jobs.size() - wv.chain_lo; wv.wf_n = (int)wf_jobs.size() - wv.wf_lo;
-        wv.chunk_n = (int)mb_chunks.size() - wv.chunk_lo; wv.kw_n = (int)kw_jobs.size() - wv.kw_lo;
-        wv.gain_n = (int)gain_jobs.size() - wv.gain_lo; wv.seg_hi = n_seg_total;
-        wv.lim_n = (int)lim_jobs.size() - wv.lim_lo;
-        for (int t = wv.track_lo; t < wv.track_hi; ++t) {
-            wv.limiter = wv.limiter || (p->tracks[t].flags & AME_F_LIMITER);
-            wv.true_peak = wv.true_peak || (p->tracks[t].flags & AME_F_TRUE_PEAK);
-        }
-        p->slot_lim_jobs = std::max(p->slot_lim_jobs, wv.lim_n);
-        p->slot_tiles = std::max(p->slot_tiles, wv.wf_n);
-        p->slot_chains = std::max(p->slot_chains, wv.chain_n);
+    // ---- layout: tiles are sized for the resident 128-thread CTAs of k_eq and k_band_split -------------
+    DeviceShape shape{148, 2, 3};
+    cudaDeviceGetAttribute(&shape.n_sm, cudaDevAttrMultiProcessorCount, device);
+    if (p->precision == 1) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shape.occ_eq, k_eq_f32, 128, 0);
+    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shape.occ_eq, k_eq, 128, 0);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shape.occ_split, k_band_split<true>, 128, 0);
+    p->n_sm = shape.n_sm;
+    JobTables jobs;
+    std::string err;
+    int rc = build_layout(tracks, n_tracks, o, shape, *p, jobs, err);
+    if (rc) {
+        g_err = err;
+        return bail(rc);
     }
 
     // ---- device state -------------------------------------------------------------------------
-    if ((rc = upload(&p->d_tracks, p->tracks)) || (rc = upload(&p->d_tdev, p->tdev)) || (rc = upload(&p->d_mb_delta, mb_delta)) ||
-        (rc = upload(&p->d_eq_jobs, eq_jobs)) || (rc = upload(&p->d_split_jobs, split_jobs)) ||
-        (rc = upload(&p->d_chain_jobs, chain_jobs)) || (rc = upload(&p->d_wf_jobs, wf_jobs)) || (rc = upload(&p->d_mb_chunks, mb_chunks)) ||
-        (rc = upload(&p->d_kw_jobs, kw_jobs)) || (rc = upload(&p->d_gain_jobs, gain_jobs)) || (rc = upload(&p->d_lim_jobs, lim_jobs)) || (rc = upload(&p->d_tables, tables)))
+    if ((rc = upload(p, &p->d_tracks, p->tracks)) || (rc = upload(p, &p->d_tdev, p->tdev)) || (rc = upload(p, &p->d_mb_delta, jobs.mb_delta)) ||
+        (rc = upload(p, &p->d_eq_jobs, jobs.eq)) || (rc = upload(p, &p->d_split_jobs, jobs.split)) ||
+        (rc = upload(p, &p->d_chain_jobs, jobs.chain)) || (rc = upload(p, &p->d_wf_jobs, jobs.wf)) ||
+        (rc = upload(p, &p->d_mb_chunks, jobs.mb_chunks)) || (rc = upload(p, &p->d_kw_jobs, jobs.kw)) ||
+        (rc = upload(p, &p->d_gain_jobs, jobs.gain)) || (rc = upload(p, &p->d_lim_jobs, jobs.lim)) || (rc = upload(p, &p->d_tables, jobs.att)))
         return bail(rc);
     const size_t fb = (size_t)p->total_frames * 4;
-    p->slots.resize(n_slots);
+    p->slots.resize(p->n_slots);
     for (Slot &sl : p->slots) {
         if ((rc = dmalloc(p, (void **)&sl.pre, (size_t)p->slot_frames * 4)) ||
             (rc = dmalloc(p, (void **)&sl.bands, (size_t)p->mb_frames * 4 * 3)) ||
@@ -1050,7 +527,7 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
             (p->mb_frames && cudaMemsetAsync(sl.bands, 0, (size_t)p->mb_frames * 12, 0) != cudaSuccess))
             return bail(fail(AME_E_CUDA, "cudaMemset failed"));
     }
-    if ((rc = dmalloc(p, (void **)&p->d_chain_stats, std::max<size_t>(chain_jobs.size(), 1) * 2 * sizeof(int))) ||
+    if ((rc = dmalloc(p, (void **)&p->d_chain_stats, std::max<size_t>(jobs.chain.size(), 1) * 2 * sizeof(int))) ||
         (rc = dmalloc(p, (void **)&p->d_energy, (size_t)std::max<int64_t>(p->n_sb_total, 1) * 8)) ||
         (rc = dmalloc(p, (void **)&p->d_hist, (size_t)n_tracks * 1000 * 8)) ||
         (rc = dmalloc(p, (void **)&p->d_hist_st, (size_t)n_tracks * 1000 * 4)) ||
@@ -1060,7 +537,7 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
         (rc = dmalloc(p, (void **)&p->d_results, (size_t)n_tracks * sizeof(ame_track_result))))
         return bail(rc);
     if (cudaMemsetAsync(p->d_lim_stats, 0, 4 * sizeof(int), 0) != cudaSuccess) return bail(fail(AME_E_CUDA, "cudaMemset failed"));
-    if (cudaMemsetAsync(p->d_chain_stats, 0, std::max<size_t>(chain_jobs.size(), 1) * 2 * sizeof(int), 0) != cudaSuccess)
+    if (cudaMemsetAsync(p->d_chain_stats, 0, std::max<size_t>(jobs.chain.size(), 1) * 2 * sizeof(int), 0) != cudaSuccess)
         return bail(fail(AME_E_CUDA, "cudaMemset failed"));
     if (o.host_io) {
         if ((rc = dmalloc(p, (void **)&p->d_in, fb)) || (rc = dmalloc(p, (void **)&p->d_out, fb))) return bail(rc);
@@ -1072,6 +549,7 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
             cudaStreamCreateWithFlags(&p->s_out, cudaStreamNonBlocking) != cudaSuccess)
             return bail(fail(AME_E_CUDA, "cudaStreamCreate failed"));
     }
+    const int n_waves = (int)p->waves.size();
     if (o.host_io || n_waves > 1) {
         p->ev_in.resize(n_waves);
         p->ev_run.resize(n_waves);
@@ -1113,6 +591,7 @@ int ame_plan_set_warm_luts(ame_plan *p, const float *luts, int32_t n_luts) {
     GUARD(p->device);
     if (p->d_luts) {
         CU(cudaDeviceSynchronize());
+        p->allocs.erase(std::find(p->allocs.begin(), p->allocs.end(), (void *)p->d_luts));
         dev_free(p->d_luts);
         p->d_luts = nullptr;
         p->ws_bytes -= (size_t)p->n_luts * 65536 * sizeof(double);
@@ -1154,7 +633,7 @@ int ame_plan_chain_stats(ame_plan *p, int64_t *n_chains, int64_t *steps, int64_t
     GUARD(p->device);
     CU(cudaDeviceSynchronize());
     int64_t nc = 0;
-    for (const Wave &w : p->waves) nc += w.chain_n;
+    for (const Wave &w : p->waves) nc += w.chain.n;
     std::vector<int> h((size_t)std::max<int64_t>(nc, 1) * 2, 0);
     if (nc) CU(cudaMemcpy(h.data(), p->d_chain_stats, (size_t)nc * 2 * sizeof(int), cudaMemcpyDeviceToHost));
     int64_t st = 0, mx = 0, ps = 0;
@@ -1262,7 +741,7 @@ int ame_stage_band_split(ame_plan *p, const int16_t *d_pre, int16_t *d_bands, vo
     if (!p || !d_pre) return fail(AME_E_INVALID, "NULL argument");
     SINGLE_WAVE(p);
     GUARD(p->device);
-    if (p->waves[0].split_n && !d_bands) return fail(AME_E_INVALID, "NULL bands buffer");
+    if (p->waves[0].split.n && !d_bands) return fail(AME_E_INVALID, "NULL bands buffer");
     return run_split(p, p->waves[0], d_pre, d_bands, (cudaStream_t)stream);
 }
 
@@ -1270,7 +749,7 @@ int ame_stage_compress(ame_plan *p, int16_t *d_bands, int16_t *d_pre, void *stre
     if (!p || !d_pre) return fail(AME_E_INVALID, "NULL argument");
     SINGLE_WAVE(p);
     GUARD(p->device);
-    if (p->waves[0].chain_n && !d_bands) return fail(AME_E_INVALID, "NULL bands buffer");
+    if (p->waves[0].chain.n && !d_bands) return fail(AME_E_INVALID, "NULL bands buffer");
     Bufs b = slot_bufs(p, p->waves[0], nullptr, nullptr);
     b.bands = d_bands;
     b.pre = d_pre;

@@ -12,51 +12,11 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include "../../include/ame.h"
+#include "ame_layout.h"
 
 namespace ame {
 
-constexpr int kGainTile = 32768;   // frames per CTA in k_apply_gain / k_band_sum
 constexpr unsigned kFull = 0xffffffffu;
-
-struct TileJob {           // one lane pair of k_eq / k_band_split
-    int64_t chunk_begin;   // absolute frame index (packed buffer) where filter state is reset
-    int64_t tile_begin;    // first frame this job writes (absolute, multiple of 4 unless == chunk_begin)
-    int64_t tile_end;      // one past the last frame it writes
-    int32_t track;
-    int32_t variant;       // EQ stage mask (bit s = stage s active)
-};
-
-struct ChainJob {          // one warp of k_compress: one band of one chunk of a multiband track
-    int64_t mb_begin;      // of the chunk, in the multiband-only packing (bands planes)
-    int64_t n;             // frames
-    int64_t grp_begin;     // first slot of this chain in the per-group record array
-    int32_t band;
-    int32_t table;
-    uint32_t thr_i;        // rms > thresh_rms  <=>  rms >= thr_i
-    int32_t look;          // look_frames
-    int32_t tile0;         // index (within the wave's launch) of the chain's first k_window_flag / k_compact tile
-    int32_t pad;
-};
-
-struct KwJob { int32_t track; int32_t sb_begin; int32_t sb_end; int32_t pad; };
-
-struct GainJob { int64_t begin; int64_t end; int32_t track; int32_t pad; };
-
-// indexed by integer rms 0..32768.  tau = the smallest attenuation a with fl(a + inc) >= m, so that
-// (att + inc < m) <=> (att < tau) exactly and the branch predicates depend on the OLD attenuation only.
-struct AttEntry { double m, inc, dec, tau; };
-
-struct TrackDev {          // device-side per-track bookkeeping
-    int64_t sb_offset;     // start of this track's 100 ms energies in the energy array
-    int32_t n_sb;          // number of complete 100 ms sub-blocks (halo included)
-    int32_t s100;          // frames per 100 ms = (fs + 5) / 10   (ebur128.c)
-    int32_t first_block;   // time shards: 400 ms blocks before this one belong to the previous shard / the warm-up
-    int32_t lim_tile0;     // limiter: index (within the wave's launch) of the track's first limiter tile
-    int64_t n_total;       // halo + span frames
-    int32_t lim_shift;     // limiter: log2 of the track's limiter tile length (a power of two >= G)
-    int32_t pad;
-};
 
 __constant__ double c_hist_bounds[1001];
 __constant__ double c_hist_energy[1000];
@@ -331,8 +291,6 @@ AME_EQ_KERNEL(k_eq_f32, float, false)      // precision experiment only (ame_pla
 // truncated to int16 (apply_multiband_compressor :300-305).  One thread per tile, both channels, same
 // warm-up scheme.  bands = 3 planes of mb_frames frames each.
 // ------------------------------------------------------------------------------------------------
-struct XoverCfg { double lb0, la10, la20, la11, la21, hb0, ha10, ha20, ha11, ha21; };
-
 // UNI: every multiband track of the launch has the same crossover (same sample rate) - the usual case; the
 // coefficients then come from the kernel parameter and live in uniform registers.
 template <bool UNI>
@@ -431,33 +389,6 @@ k_band_split(const __grid_constant__ XoverCfg xc, const TileJob *__restrict__ jo
 // only flagged frames take the square root (S/n is never within 2^-41 of a perfect square unless equal,
 // hence the double-precision expression of audioop truncates to the exact integer root).
 // ------------------------------------------------------------------------------------------------
-constexpr int kWfThreads = 256;
-constexpr int kWfTile = 2048;      // frames per CTA of k_window_flag / k_compact (8 per thread)
-constexpr int kSeg = 256;          // frames per k_att_chain iteration / per k_compress_apply warp (8 groups)
-
-// One tile of a chain for k_window_flag / k_compact.  It carries what the kernels need of its chain, so a CTA (which
-// lives for a few microseconds) starts with ONE dependent load instead of job -> chain -> data.
-struct WfJob {
-    int64_t tile_begin;    // relative to the chunk
-    int64_t plane_off;     // band * mb_frames + mb_begin: offset of the chain in the bands / rms / list planes (frames)
-    int64_t n;             // frames of the chain
-    int64_t grp_begin;     // first group record of the chain
-    int32_t chain;         // index into the plan's chain table
-    int32_t look;          // look_frames
-    uint32_t thr_i;        // rms > thresh_rms  <=>  rms >= thr_i
-    int32_t tile0;         // index (within the launch) of the chain's first tile
-};
-
-struct MbChunk {           // one chunk of a multiband track (k_compress_apply)
-    int64_t abs_begin;     // absolute frame index in the packed pre buffer
-    int64_t mb_begin;      // frame index in the multiband-only packing
-    int64_t n;             // frames
-    int64_t seg_prefix;    // kSeg-segments in all earlier chunks
-    int64_t grp_begin[3];  // first group record of each band's chain
-    int32_t track;
-    int32_t pad;
-};
-
 __device__ __forceinline__ unsigned energy_of(uint32_t w) {          // l^2 + r^2 <= 2^31
     const int l = (int16_t)(w & 0xffffu), r = (int16_t)(w >> 16);
     return (unsigned)(l * l) + (unsigned)(r * r);
@@ -484,8 +415,6 @@ __device__ __forceinline__ unsigned isqrt_ratio(unsigned long long s, unsigned n
     else if ((unsigned long long)(r + 1) * (r + 1) * n <= s) ++r;
     return r;
 }
-
-struct GrpRec { uint32_t mask, base; };   // per 32-frame group of a chain: flagged frames, flagged frames before the group
 
 __global__ void __launch_bounds__(kWfThreads)
 k_window_flag(const WfJob *__restrict__ jobs, const int16_t *__restrict__ bands, uint16_t *__restrict__ rms,
@@ -632,8 +561,6 @@ __device__ __forceinline__ double att_update(double att, double m, double inc, d
 // The walk is a software pipeline: rms values two 8-step blocks ahead, table entries (one 32-byte gather per step)
 // one block ahead, 25 cycles per dependent step (profiles/micro/att_chain_latency3.cu).
 // ------------------------------------------------------------------------------------------------
-constexpr int kChainMaxThreads = 256;
-
 struct RmsBlk { uint32_t w[4]; };         // 8 consecutive entries of the dense rms list
 
 // entries [i, i+8) of the list, entries at or past `lim` read as 0 (= the no-op table entry)
@@ -994,8 +921,6 @@ k_compress_apply(const MbChunk *__restrict__ chunks, int n_chunks, int64_t seg_l
 // whole track (the reference measures the concatenated file), so warm-up may cross chunk joins.
 // One thread per tile of sub-blocks, both channels (two independent chains).
 // ------------------------------------------------------------------------------------------------
-struct KwCfg { double b0, b1, b2, a1, a2, ra1, ra2; };   // pre-filter biquad; RLB denominators (numerator 1 -2 1)
-
 // UNI: every track of the launch has the same K filter (same sample rate): coefficients from the kernel parameter.
 template <bool UNI>
 __global__ void __launch_bounds__(128, 5)
@@ -1278,8 +1203,6 @@ k_apply_gain(const GainJob *__restrict__ jobs, const ame_track_result *__restric
 // One warp per non-elementwise tile: lane 0 walks the state 32 frames at a time, all lanes load the frames before and
 // scale / round / store them after.
 // ------------------------------------------------------------------------------------------------
-constexpr int kLimQueue = 1024;     // largest queue capacity (look-ahead B <= 1000 frames is validated by the host)
-
 // The machine between two frames, as recorded per tile.  The queue (one entry per over-limit frame still inside the
 // look-ahead ring: up to B of them while the signal clips) lives in two side arrays of `keep` = B_max + 2 entries per tile.
 struct LimState {

@@ -1,5 +1,5 @@
 """k_eq time per stereo frame for every template variant the C4 sweep uses (and a few more), each as a batch of
-identical tracks - the data behind eq_cost_per_frame() in csrc/ame.cu (tiles are sized so that every thread of a launch
+identical tracks - the data behind eq_cost_per_frame() in csrc/ame_layout.h (tiles are sized so that every thread of a launch
 does the same amount of work; a wrong relative cost leaves the cheap tracks' warps idle at the end of the launch)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))

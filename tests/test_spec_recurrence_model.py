@@ -14,7 +14,7 @@ from oracle import chain
 
 
 def _entries(fs, threshold, ratio):
-    """(M, inc, dec, tau) per integer rms, as build_att_table in csrc/ame.cu does; flagged(r) = r > thresh_rms."""
+    """(M, inc, dec, tau) per integer rms, as build_att_table in csrc/ame_layout.h does; flagged(r) = r > thresh_rms."""
     thr, _look, attack_frames, release_frames = chain.compressor_constants(fs, threshold, ratio)
     table = {}
 
