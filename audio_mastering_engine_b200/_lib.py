@@ -8,6 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libame.so")
 
 AME_F_WARMTH, AME_F_WIDTH, AME_F_MULTIBAND, AME_F_NORMALIZE, AME_F_LIMITER, AME_F_TRUE_PEAK = 1, 2, 4, 8, 16, 32
+AME_F_MEASURE_OUTPUT = 64
 AME_N_KERNELS = 12
 AME_EQ_BYPASS, AME_EQ_SHELF_BOOST, AME_EQ_SHELF_CUT, AME_EQ_PEAK = 0, 1, 2, 3
 AME_ABI_VERSION = 5
@@ -46,6 +47,12 @@ class TrackResult(C.Structure):
                 ("true_peak", C.c_double)]
 
 
+class Loudness(C.Structure):
+    _fields_ = [("integrated", C.c_double), ("thresh", C.c_double), ("lra", C.c_double), ("true_peak", C.c_double),
+                ("max_momentary", C.c_double), ("max_short_term", C.c_double), ("n_blocks", C.c_int64),
+                ("sample_peak", C.c_int32), ("measured", C.c_int32)]
+
+
 class PlanOptions(C.Structure):
     _fields_ = [("eq_tile_frames", C.c_int32), ("xover_tile_frames", C.c_int32), ("kw_tile_subblocks", C.c_int32),
                 ("host_io", C.c_int32), ("n_waves", C.c_int32), ("chain_warps", C.c_int32), ("n_slots", C.c_int32),
@@ -64,6 +71,7 @@ SYMBOLS = {
     "ame_sizeof_track_params": (C.c_size_t, []),
     "ame_sizeof_track_result": (C.c_size_t, []),
     "ame_sizeof_plan_options": (C.c_size_t, []),
+    "ame_sizeof_loudness": (C.c_size_t, []),
     "ame_last_error": (C.c_char_p, []),
     "ame_device_count": (C.c_int, [C.POINTER(C.c_int)]),
     "ame_release_cached_memory": (C.c_int, [C.c_int]),
@@ -85,6 +93,8 @@ SYMBOLS = {
     "ame_plan_kernel_timeline": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_float), C.c_int]),
     "ame_master_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(TrackResult), C.c_void_p]),
     "ame_master_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(TrackResult)]),
+    "ame_plan_output_loudness": (C.c_int, [C.c_void_p, C.POINTER(Loudness), C.c_void_p]),
+    "ame_measure_loudness": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(Loudness), C.c_void_p]),
     "ame_measure_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ame_normalize_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(TrackResult), C.c_void_p]),
     "ame_shard_halo_exchange": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_void_p]),
@@ -118,7 +128,7 @@ def load():
             fn.restype = res
             fn.argtypes = args
         if (lib.ame_sizeof_track_params() != C.sizeof(TrackParams) or lib.ame_sizeof_track_result() != C.sizeof(TrackResult)
-                or lib.ame_sizeof_plan_options() != C.sizeof(PlanOptions)):
+                or lib.ame_sizeof_plan_options() != C.sizeof(PlanOptions) or lib.ame_sizeof_loudness() != C.sizeof(Loudness)):
             raise AmeError("ctypes structs are out of sync with include/ame.h")
         if lib.ame_abi_version() != AME_ABI_VERSION:
             raise AmeError(f"libame.so has ABI version {lib.ame_abi_version()}, this package needs {AME_ABI_VERSION}: "

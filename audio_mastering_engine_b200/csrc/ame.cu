@@ -3,6 +3,7 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
+#include <cstring>
 #include <dlfcn.h>
 #include <mutex>
 #include <string>
@@ -157,8 +158,19 @@ struct ame_plan : Layout {
     unsigned *d_tp = nullptr;               // per track: float bits of the oversampled peak (k_true_peak)
     int *d_lim_stats = nullptr;             // open tiles after the limiter's round 0 / 1 / 2, accumulated
     ame_track_result *d_results = nullptr;
+    // output meter (tracks with AME_F_MEASURE_OUTPUT; none of it exists without such a track)
+    KwJob *d_meter_kw = nullptr;
+    GainJob *d_meter_peak = nullptr;
+    int32_t *d_meter_tracks = nullptr;
+    TrackDev *d_meter_tdev = nullptr;
+    double *d_meter_energy = nullptr;       // sub-block energies of the flagged tracks (meter_tdev[t].sb_offset)
+    int *d_meter_sp = nullptr;              // per track: sample peak
+    unsigned *d_meter_tp = nullptr;         // per track: float bits of the oversampled peak
+    ame_loudness *d_loud_out = nullptr;     // per track: meter of the last ame_master_* / ame_normalize_device call
+    ame_loudness *d_loud_any = nullptr;     // per track: the last ame_measure_loudness
     cudaStream_t s_in = nullptr, s_out = nullptr;                       // host path: copy-in / copy-out
     std::vector<cudaEvent_t> ev_in, ev_run;                             // per wave
+    std::vector<cudaEvent_t> ev_meter;                                  // host path with the meter: per slot, its last meter done
     // optional per-kernel CUDA-event timing (ame_plan_set_timing)
     bool timing = false;
     int t_step = -1, t_wave = 0;
@@ -402,6 +414,31 @@ int run_gain(ame_plan *p, const Wave &w, const int16_t *d_pre, const int64_t *d_
     return run_apply(p, w, d_pre, d_out, b, s);
 }
 
+// the output meter over the flagged tracks of wave w, read from `buf` (absolute packed-buffer addressing), into `res`
+int run_meter(ame_plan *p, const Wave &w, const int16_t *buf, ame_loudness *res, cudaStream_t s) {
+    if (!w.meter_tracks.n) return AME_OK;
+    const int nt = w.track_hi - w.track_lo;
+    CU(cudaMemsetAsync(p->d_meter_sp + w.track_lo, 0, (size_t)nt * 4, s));
+    CU(cudaMemsetAsync(p->d_meter_tp + w.track_lo, 0, (size_t)nt * 4, s));
+    if (w.meter_kw.n) {
+        if (w.kw_uni)
+            k_kweight_energy<true><<<(w.meter_kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_meter_kw + w.meter_kw.lo, w.meter_kw.n, p->d_tracks,
+                                                                              p->d_meter_tdev, buf, p->d_meter_energy, p->d_meter_sp);
+        else
+            k_kweight_energy<false><<<(w.meter_kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_meter_kw + w.meter_kw.lo, w.meter_kw.n, p->d_tracks,
+                                                                               p->d_meter_tdev, buf, p->d_meter_energy, p->d_meter_sp);
+        LAUNCH_CHECK(p);
+    }
+    if (w.meter_peak.n) {
+        k_meter_peak<<<w.meter_peak.n, 256, 0, s>>>(p->d_meter_peak + w.meter_peak.lo, p->d_tracks, buf, p->d_meter_tp, p->d_meter_sp);
+        LAUNCH_CHECK(p);
+    }
+    k_meter_finalize<<<w.meter_tracks.n, 256, 0, s>>>(p->d_meter_tracks + w.meter_tracks.lo, p->d_tracks, p->d_meter_tdev, p->d_meter_energy,
+                                                      p->d_meter_sp, p->d_meter_tp, res);
+    LAUNCH_CHECK(p);
+    return AME_OK;
+}
+
 int run_measure(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     int rc;
     if ((rc = run_eq(p, w, b.in, b.pre, s))) return rc;
@@ -431,6 +468,7 @@ int ame_abi_version(void) { return AME_ABI_VERSION; }
 size_t ame_sizeof_track_params(void) { return sizeof(ame_track_params); }
 size_t ame_sizeof_track_result(void) { return sizeof(ame_track_result); }
 size_t ame_sizeof_plan_options(void) { return sizeof(ame_plan_options); }
+size_t ame_sizeof_loudness(void) { return sizeof(ame_loudness); }
 const char *ame_last_error(void) { return g_err.c_str(); }
 const char *ame_kernel_name(int slot) { return (slot >= 0 && slot < AME_N_KERNELS) ? kKernelNames[slot] : ""; }
 
@@ -452,6 +490,7 @@ void ame_plan_destroy(ame_plan *p) {
         if (s) cudaStreamDestroy(s);
     for (cudaEvent_t e : p->ev_in) cudaEventDestroy(e);
     for (cudaEvent_t e : p->ev_run) cudaEventDestroy(e);
+    for (cudaEvent_t e : p->ev_meter) cudaEventDestroy(e);
     for (cudaEvent_t e : p->t_ev) cudaEventDestroy(e);
     for (cudaEvent_t e : p->tl_ev) cudaEventDestroy(e);
     delete p;
@@ -498,6 +537,10 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
         (rc = upload(p, &p->d_mb_chunks, jobs.mb_chunks)) || (rc = upload(p, &p->d_kw_jobs, jobs.kw)) ||
         (rc = upload(p, &p->d_gain_jobs, jobs.gain)) || (rc = upload(p, &p->d_lim_jobs, jobs.lim)) || (rc = upload(p, &p->d_tables, jobs.att)))
         return bail(rc);
+    if (p->any_meter &&
+        ((rc = upload(p, &p->d_meter_kw, jobs.meter_kw)) || (rc = upload(p, &p->d_meter_peak, jobs.meter_peak)) ||
+         (rc = upload(p, &p->d_meter_tracks, jobs.meter_tracks)) || (rc = upload(p, &p->d_meter_tdev, p->meter_tdev))))
+        return bail(rc);
     const size_t fb = (size_t)p->total_frames * 4;
     p->slots.resize(p->n_slots);
     for (Slot &sl : p->slots) {
@@ -537,6 +580,17 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
         (rc = dmalloc(p, (void **)&p->d_results, (size_t)n_tracks * sizeof(ame_track_result))))
         return bail(rc);
     if (cudaMemsetAsync(p->d_lim_stats, 0, 4 * sizeof(int), 0) != cudaSuccess) return bail(fail(AME_E_CUDA, "cudaMemset failed"));
+    if (p->any_meter) {
+        const size_t lb = (size_t)n_tracks * sizeof(ame_loudness);
+        if ((rc = dmalloc(p, (void **)&p->d_meter_energy, (size_t)std::max<int64_t>(p->meter_sb_total, 1) * 8)) ||
+            (rc = dmalloc(p, (void **)&p->d_meter_sp, (size_t)n_tracks * 4)) ||
+            (rc = dmalloc(p, (void **)&p->d_meter_tp, (size_t)n_tracks * 4)) ||
+            (rc = dmalloc(p, (void **)&p->d_loud_out, lb)) || (rc = dmalloc(p, (void **)&p->d_loud_any, lb)))
+            return bail(rc);
+        // measured = 0 everywhere until a call meters
+        if (cudaMemsetAsync(p->d_loud_out, 0, lb, 0) != cudaSuccess || cudaMemsetAsync(p->d_loud_any, 0, lb, 0) != cudaSuccess)
+            return bail(fail(AME_E_CUDA, "cudaMemset failed"));
+    }
     if (cudaMemsetAsync(p->d_chain_stats, 0, std::max<size_t>(jobs.chain.size(), 1) * 2 * sizeof(int), 0) != cudaSuccess)
         return bail(fail(AME_E_CUDA, "cudaMemset failed"));
     if (o.host_io) {
@@ -560,6 +614,11 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
             if (cudaEventCreateWithFlags(&p->ev_in[w], cudaEventDisableTiming) != cudaSuccess ||
                 cudaEventCreateWithFlags(&p->ev_run[w], cudaEventDisableTiming) != cudaSuccess)
                 return bail(fail(AME_E_CUDA, "cudaEventCreate failed"));
+        if (o.host_io && p->any_meter) {
+            p->ev_meter.resize(p->slots.size());
+            for (cudaEvent_t &e : p->ev_meter)
+                if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return bail(fail(AME_E_CUDA, "cudaEventCreate failed"));
+        }
     }
 
     // ebur128.c histogram tables (same libm calls as the C library)
@@ -821,6 +880,7 @@ int ame_normalize_device(ame_plan *p, const int64_t *d_hist, int16_t *d_out, ame
         p->t_wave = (int)std::min<size_t>(w, kMaxTimedWaves - 1);
         const Bufs b = slot_bufs(p, p->waves[w], nullptr, d_out);
         if ((rc = run_gain(p, p->waves[w], b.pre, d_hist, d_out, b, s))) return rc;
+        if ((rc = run_meter(p, p->waves[w], d_out, p->d_loud_out, s))) return rc;
     }
     if (results) {
         CU(cudaMemcpyAsync(results, p->d_results, (size_t)p->n_tracks * sizeof(ame_track_result), cudaMemcpyDeviceToHost, s));
@@ -921,6 +981,7 @@ int ame_master_device(ame_plan *p, const int16_t *d_in, int16_t *d_out, ame_trac
     if (nw <= 1) {
         p->t_wave = 0;
         if ((rc = run_chain_of_stages(p, p->waves[0], slot_bufs(p, p->waves[0], d_in, d_out), s))) return rc;
+        if ((rc = run_meter(p, p->waves[0], d_out, p->d_loud_out, s))) return rc;
     } else {
         // several waves: fork the caller's stream into the slots' streams and join again.  Waves of different slots
         // overlap (the latency-bound compressor kernels of one under the FP64-bound filters of another); waves of
@@ -932,6 +993,7 @@ int ame_master_device(ame_plan *p, const int16_t *d_in, int16_t *d_out, ame_trac
             if (w < ns) CU(cudaStreamWaitEvent(ws, p->ev_in[0], 0));
             p->t_wave = std::min(w, kMaxTimedWaves - 1);
             if ((rc = run_chain_of_stages(p, p->waves[w], slot_bufs(p, p->waves[w], d_in, d_out), ws))) return drain(p, rc);
+            if ((rc = run_meter(p, p->waves[w], d_out, p->d_loud_out, ws))) return drain(p, rc);
         }
         for (int k = 0; k < ns; ++k) {
             CU(cudaEventRecord(p->ev_run[k], p->slots[k].stream));
@@ -979,6 +1041,8 @@ static int master_host_impl(ame_plan *p, const int16_t *h_in, int16_t *h_out, am
         if ((rc = run_chain_of_stages(p, p->waves[w], slot_bufs(p, p->waves[w], p->d_in, p->d_out), ws))) return rc;
         CU(cudaEventRecord(p->ev_run[w], ws));
         if (tl) CU(cudaEventRecord(p->tl_ev[3 + 4 * w], ws));
+        // the meter reads d_out after ev_run[w]: the wave's D2H copy waits for its kernels, not for its meter
+        if ((rc = run_meter(p, p->waves[w], p->d_out, p->d_loud_out, ws))) return rc;
     }
     for (int w = 0; w < nw; ++w) {
         const Wave &wv = p->waves[w];
@@ -989,7 +1053,43 @@ static int master_host_impl(ame_plan *p, const int16_t *h_in, int16_t *h_out, am
     }
     if (results)
         CU(cudaMemcpyAsync(results, p->d_results, (size_t)p->n_tracks * sizeof(ame_track_result), cudaMemcpyDeviceToHost, p->s_out));
+    // only now, behind every copy, s_out waits for the meters of all slots: the synchronisation below covers them
+    if (p->any_meter)
+        for (size_t k = 0; k < p->slots.size(); ++k) {
+            CU(cudaEventRecord(p->ev_meter[k], p->slots[k].stream));
+            CU(cudaStreamWaitEvent(p->s_out, p->ev_meter[k], 0));
+        }
     CU(cudaStreamSynchronize(p->s_out));
+    return AME_OK;
+}
+
+int ame_plan_output_loudness(ame_plan *p, ame_loudness *out, void *stream) {
+    if (!p || !out) return fail(AME_E_INVALID, "NULL argument");
+    GUARD(p->device);
+    if (!p->any_meter) {                               // nothing is ever measured
+        std::memset(out, 0, (size_t)p->n_tracks * sizeof(ame_loudness));
+        return AME_OK;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    CU(cudaMemcpyAsync(out, p->d_loud_out, (size_t)p->n_tracks * sizeof(ame_loudness), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    return AME_OK;
+}
+
+int ame_measure_loudness(ame_plan *p, const int16_t *d_buf, ame_loudness *out, void *stream) {
+    if (!p || !d_buf) return fail(AME_E_INVALID, "NULL argument");
+    if (!p->any_meter) return fail(AME_E_INVALID, "no track carries AME_F_MEASURE_OUTPUT");
+    GUARD(p->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    p->launches = 0;
+    CU(cudaMemsetAsync(p->d_loud_any, 0, (size_t)p->n_tracks * sizeof(ame_loudness), s));
+    int rc;
+    for (const Wave &w : p->waves)
+        if ((rc = run_meter(p, w, d_buf, p->d_loud_any, s))) return rc;
+    if (out) {
+        CU(cudaMemcpyAsync(out, p->d_loud_any, (size_t)p->n_tracks * sizeof(ame_loudness), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+    }
     return AME_OK;
 }
 

@@ -1054,9 +1054,65 @@ k_block_hist(const TrackDev *__restrict__ tdev, int track_lo, const double *__re
     }
 }
 
+// ebur128_gated_loudness over a 400 ms block histogram, in ebur128.c's order (the sums are order-sensitive in the last
+// bit, and that bit can decide the '%.2f' the gain is made of): blocks above the absolute gate, the relative gate (as
+// energy and in LUFS; -70 when no block passes) and the gated loudness (-inf when no block passes the relative gate).
+// k_finalize and k_meter_finalize both walk with it.
+struct GateWalk { long long count, above; double rel, thresh, integrated; };
+template <class H>
+__device__ __forceinline__ GateWalk gate_walk(const H *h) {
+    GateWalk g{0, 0, 0.0, -70.0, -INFINITY};
+    double rel = 0.0; long long count = 0;
+    for (int j = 0; j < 1000; ++j) { rel += (double)h[j] * c_hist_energy[j]; count += h[j]; }
+    g.count = count;
+    if (count > 0) {
+        rel /= (double)count;
+        rel *= 0.1;                                  // RELATIVE_GATE_FACTOR = 10^(-10/10)
+        g.rel = rel;
+        g.thresh = 10.0 * log10(rel) - 0.691;        // ff_ebur128_relative_threshold
+        int start;
+        if (rel < c_hist_bounds[0]) start = 0;
+        else { start = hist_index(rel); if (rel > c_hist_energy[start]) ++start; }
+        double gated = 0.0; long long above = 0;
+        for (int j = start; j < 1000; ++j) { gated += (double)h[j] * c_hist_energy[j]; above += h[j]; }
+        g.above = above;
+        if (above > 0) {
+            gated /= (double)above;
+            g.integrated = 10.0 * log10(gated) - 0.691;
+        }
+    }
+    return g;
+}
+
+// ff_ebur128_loudness_range over a short-term histogram: blocks above (mean power - 20 dB), 10th .. 95th percentile; 0
+// when there is none
+template <class HS>
+__device__ __forceinline__ double lra_walk(const HS *hs) {
+    long long n = 0; double power = 0.0;
+    for (int j = 0; j < 1000; ++j) { n += hs[j]; power += (double)hs[j] * c_hist_energy[j]; }
+    if (n > 0) {
+        power /= (double)n;
+        const double integ = 0.01 * power;           // MINUS_20DB
+        int idx;
+        if (integ < c_hist_bounds[0]) idx = 0;
+        else { idx = hist_index(integ); if (integ > c_hist_energy[idx]) ++idx; }
+        long long m = 0;
+        for (int j = idx; j < 1000; ++j) m += hs[j];
+        if (m > 0) {
+            const long long p_lo = (long long)((double)(m - 1) * 0.1 + 0.5), p_hi = (long long)((double)(m - 1) * 0.95 + 0.5);
+            long long acc = 0; int j = idx;
+            while (acc <= p_lo) acc += hs[j++];
+            const double l_en = c_hist_energy[j - 1];
+            while (acc <= p_hi) acc += hs[j++];
+            const double h_en = c_hist_energy[j - 1];
+            return (10.0 * log10(h_en) - 0.691) - (10.0 * log10(l_en) - 0.691);
+        }
+    }
+    return 0.0;
+}
+
 // k_finalize: ebur128_gated_loudness + loudness range + the linear-mode gain of af_loudnorm.  One CTA per track: the
-// two 1000-bin histograms are staged in shared memory by all threads, then ONE thread walks them in the order
-// ebur128.c does (the sums are order-sensitive in the last bit, and that bit can decide the '%.2f' the gain is made of).
+// two 1000-bin histograms are staged in shared memory by all threads, then ONE thread walks them.
 __global__ void __launch_bounds__(128)
 k_finalize(const ame_track_params *__restrict__ tracks, int track_lo, int track_hi,
            const long long *__restrict__ hist, const int *__restrict__ hist_st, const int *__restrict__ peak,
@@ -1071,29 +1127,19 @@ k_finalize(const ame_track_params *__restrict__ tracks, int track_lo, int track_
     }
     __syncthreads();
     if (threadIdx.x != 0) return;
-    const long long *h = s_h;
     ame_track_result r;
     r.input_i = -INFINITY; r.measured_i_2dp = -INFINITY; r.gain = 1.0; r.rel_threshold = 0.0;
     r.n_blocks = 0; r.normalized = 0; r.sample_peak = peak[t];
     r.input_lra = 0.0; r.input_thresh = -70.0;
     r.true_peak = ((tracks[t].flags & AME_F_TRUE_PEAK) && tracks[t].sample_rate < 192000) ? (double)__uint_as_float(tp_bits[t])
                                                                                            : (double)peak[t] * (1.0 / 32768.0);
-    double rel = 0.0; long long count = 0;
-    for (int j = 0; j < 1000; ++j) { rel += (double)h[j] * c_hist_energy[j]; count += h[j]; }
-    r.n_blocks = count;
-    if (count > 0) {
-        rel /= (double)count;
-        rel *= 0.1;                                  // RELATIVE_GATE_FACTOR = 10^(-10/10)
-        r.rel_threshold = rel;
-        r.input_thresh = 10.0 * log10(rel) - 0.691;  // ff_ebur128_relative_threshold
-        int start;
-        if (rel < c_hist_bounds[0]) start = 0;
-        else { start = hist_index(rel); if (rel > c_hist_energy[start]) ++start; }
-        double gated = 0.0; long long above = 0;
-        for (int j = start; j < 1000; ++j) { gated += (double)h[j] * c_hist_energy[j]; above += h[j]; }
-        if (above > 0) {
-            gated /= (double)above;
-            r.input_i = 10.0 * log10(gated) - 0.691;
+    const GateWalk g = gate_walk(s_h);
+    r.n_blocks = g.count;
+    if (g.count > 0) {
+        r.rel_threshold = g.rel;
+        r.input_thresh = g.thresh;
+        if (g.above > 0) {
+            r.input_i = g.integrated;
             if (tracks[t].flags & AME_F_NORMALIZE) {
                 r.measured_i_2dp = rint(r.input_i * 100.0) / 100.0;   // the '%.2f' string of pass 1
                 r.gain = pow(10.0, (tracks[t].target_lufs - r.measured_i_2dp) / 20.0);
@@ -1101,30 +1147,7 @@ k_finalize(const ame_track_params *__restrict__ tracks, int track_lo, int track_
             }
         }
     }
-    // ff_ebur128_loudness_range: short-term blocks above (mean power - 20 dB), 10th .. 95th percentile
-    {
-        const int *hs = s_hs;
-        long long n = 0; double power = 0.0;
-        for (int j = 0; j < 1000; ++j) { n += hs[j]; power += (double)hs[j] * c_hist_energy[j]; }
-        if (n > 0) {
-            power /= (double)n;
-            const double integ = 0.01 * power;       // MINUS_20DB
-            int idx;
-            if (integ < c_hist_bounds[0]) idx = 0;
-            else { idx = hist_index(integ); if (integ > c_hist_energy[idx]) ++idx; }
-            long long m = 0;
-            for (int j = idx; j < 1000; ++j) m += hs[j];
-            if (m > 0) {
-                const long long p_lo = (long long)((double)(m - 1) * 0.1 + 0.5), p_hi = (long long)((double)(m - 1) * 0.95 + 0.5);
-                long long acc = 0; int j = idx;
-                while (acc <= p_lo) acc += hs[j++];
-                const double l_en = c_hist_energy[j - 1];
-                while (acc <= p_hi) acc += hs[j++];
-                const double h_en = c_hist_energy[j - 1];
-                r.input_lra = (10.0 * log10(h_en) - 0.691) - (10.0 * log10(l_en) - 0.691);
-            }
-        }
-    }
+    r.input_lra = lra_walk(s_hs);
     res[t] = r;
 }
 
@@ -1547,17 +1570,13 @@ __constant__ float c_tp_fir[4][12] = {
     {-0.0083007812500f, 0.0148925781250f, -0.0266113281250f, 0.0476074218750f, -0.1022949218750f, 0.9721679687500f,
      0.1373291015625f, -0.0594482421875f, 0.0332031250000f, -0.0196533203125f, 0.0109863281250f, 0.0017089843750f}};
 
-__global__ void __launch_bounds__(256)
-k_true_peak(const GainJob *__restrict__ jobs, const ame_track_params *__restrict__ tracks, const int16_t *__restrict__ pre,
-            unsigned *__restrict__ tp_bits) {
-    const GainJob job = jobs[blockIdx.x];
-    const ame_track_params *tp = tracks + job.track;
-    if (!(tp->flags & AME_F_TRUE_PEAK)) return;
+// The interpolator over one tile (GainJob) of the track that starts at frame t_begin (the frames before the tile are its
+// history), maximum |y| over both channels into the track's float bits.  k_true_peak and k_meter_peak both run it.
+__device__ __forceinline__ void true_peak_tile(const GainJob &job, const ame_track_params *tp, const uint32_t *x,
+                                               unsigned *__restrict__ tp_bits) {
     const int fs = tp->sample_rate;
-    if (fs >= 192000) return;                                          // no oversampling: k_finalize reports the sample peak
     const int step = fs < 96000 ? 1 : 2;                               // phases 0,1,2,3 (4x) or 0,2 (2x)
     const int64_t t_begin = tp->offset_frames + tp->halo_frames;
-    const uint32_t *x = reinterpret_cast<const uint32_t *>(pre);
     float best = 0.0f;
     // 8 frames per thread and iteration, 11 frames of history in front
     for (int64_t n0 = job.begin + (int64_t)threadIdx.x * 8; n0 < job.end; n0 += (int64_t)blockDim.x * 8) {
@@ -1586,6 +1605,101 @@ k_true_peak(const GainJob *__restrict__ jobs, const ame_track_params *__restrict
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) best = fmaxf(best, __shfl_xor_sync(kFull, best, d));
     if ((threadIdx.x & 31) == 0 && best > 0.0f) atomicMax(tp_bits + job.track, __float_as_uint(best));
+}
+
+__global__ void __launch_bounds__(256)
+k_true_peak(const GainJob *__restrict__ jobs, const ame_track_params *__restrict__ tracks, const int16_t *__restrict__ pre,
+            unsigned *__restrict__ tp_bits) {
+    const GainJob job = jobs[blockIdx.x];
+    const ame_track_params *tp = tracks + job.track;
+    if (!(tp->flags & AME_F_TRUE_PEAK)) return;
+    if (tp->sample_rate >= 192000) return;                             // no oversampling: k_finalize reports the sample peak
+    true_peak_tile(job, tp, reinterpret_cast<const uint32_t *>(pre), tp_bits);
+}
+
+// ------------------------------------------------------------------------------------------------
+// The output meter (AME_F_MEASURE_OUTPUT): EBU R128 over any buffer in the packed layout, for the flagged tracks of a
+// wave.  k_kweight_energy fills the meter's own sub-block energies (and the sample peak of the complete sub-blocks),
+// k_meter_peak the true peak and the sample peak of every frame, k_meter_finalize the histograms, the maxima and the
+// walk.  Every array is indexed by track, so the waves of different slots never share an entry.
+// ------------------------------------------------------------------------------------------------
+// One CTA per meter peak tile (the k_apply_gain tiles): the BS.1770 interpolator below 192 kHz (whatever the track's
+// AME_F_TRUE_PEAK), and max |s16| of every frame of the tile.
+__global__ void __launch_bounds__(256)
+k_meter_peak(const GainJob *__restrict__ jobs, const ame_track_params *__restrict__ tracks, const int16_t *__restrict__ buf,
+             unsigned *__restrict__ tp_bits, int *__restrict__ peak) {
+    const GainJob job = jobs[blockIdx.x];
+    const ame_track_params *tp = tracks + job.track;
+    const uint32_t *x = reinterpret_cast<const uint32_t *>(buf);
+    if (tp->sample_rate < 192000) true_peak_tile(job, tp, x, tp_bits);
+    int pk = 0;
+    for (int64_t f = job.begin + threadIdx.x; f < job.end; f += blockDim.x) {
+        const uint32_t w = __ldg(x + f);
+        pk = max(pk, max(abs((int)(int16_t)(w & 0xffffu)), abs((int)(int16_t)(w >> 16))));
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) pk = max(pk, __shfl_xor_sync(kFull, pk, d));
+    if ((threadIdx.x & 31) == 0 && pk > 0) atomicMax(peak + job.track, pk);
+}
+
+__device__ __forceinline__ double block_max(double v, double *s_warp) {   // over the CTA; every thread gets the result
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) v = fmax(v, __shfl_xor_sync(kFull, v, d));
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = v;
+    __syncthreads();
+    v = s_warp[0];
+    for (int i = 1; i < (int)(blockDim.x >> 5); ++i) v = fmax(v, s_warp[i]);
+    __syncthreads();
+    return v;
+}
+
+__device__ __forceinline__ double lufs_or_inf(double e) { return e >= 0.0 ? 10.0 * log10(e) - 0.691 : -INFINITY; }
+
+// One CTA of 256 threads per flagged track of the wave: both histograms in shared memory exactly as k_block_hist builds
+// them, the ungated maxima of the momentary (400 ms) and short-term (3 s) energies at every 100 ms sub-block, then ONE
+// thread walks the histograms as k_finalize does and writes the track's ame_loudness.
+__global__ void __launch_bounds__(256)
+k_meter_finalize(const int32_t *__restrict__ mtracks, const ame_track_params *__restrict__ tracks, const TrackDev *__restrict__ mtdev,
+                 const double *__restrict__ energy, const int *__restrict__ peak, const unsigned *__restrict__ tp_bits,
+                 ame_loudness *__restrict__ res) {
+    __shared__ unsigned s_hist[1000];
+    __shared__ unsigned s_st[1000];
+    __shared__ double s_warp[8];
+    const int t = mtracks[blockIdx.x];
+    for (int i = threadIdx.x; i < 1000; i += blockDim.x) { s_hist[i] = 0; s_st[i] = 0; }
+    __syncthreads();
+    const TrackDev td = mtdev[t];
+    const double *e = energy + td.sb_offset;
+    const double denom = (double)(4 * (int64_t)td.s100);
+    double mom = -1.0, st = -1.0;                    // energies are >= 0: -1 = no complete window
+    for (int j = threadIdx.x; j + 3 < td.n_sb; j += blockDim.x) {
+        const double s = (((e[j] + e[j + 1]) + e[j + 2]) + e[j + 3]) / denom;
+        mom = fmax(mom, s);
+        if (s >= c_hist_bounds[0]) atomicAdd(&s_hist[hist_index(s)], 1u);
+    }
+    // 3 s windows at every sub-block; the ones starting at a whole second are the loudness-range histogram's
+    const double denom_st = (double)(30 * (int64_t)td.s100);
+    for (int k = threadIdx.x; k + 29 < td.n_sb; k += blockDim.x) {
+        double s = 0.0;
+        for (int j = 0; j < 30; ++j) s += e[k + j];
+        s /= denom_st;
+        st = fmax(st, s);
+        if (k % 10 == 0 && s >= c_hist_bounds[0]) atomicAdd(&s_st[hist_index(s)], 1u);
+    }
+    __syncthreads();
+    mom = block_max(mom, s_warp);
+    st = block_max(st, s_warp);
+    if (threadIdx.x != 0) return;
+    ame_loudness r;
+    const GateWalk g = gate_walk(s_hist);
+    r.integrated = g.integrated; r.thresh = g.thresh; r.n_blocks = g.count;
+    r.lra = lra_walk(s_st);
+    r.sample_peak = peak[t];
+    r.true_peak = tracks[t].sample_rate < 192000 ? (double)__uint_as_float(tp_bits[t]) : (double)peak[t] * (1.0 / 32768.0);
+    r.max_momentary = lufs_or_inf(mom);
+    r.max_short_term = lufs_or_inf(st);
+    r.measured = 1;
+    res[t] = r;
 }
 
 }  // namespace ame

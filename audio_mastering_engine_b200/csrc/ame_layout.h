@@ -122,6 +122,7 @@ struct Wave {
     int track_lo = 0, track_hi = 0;
     int64_t frame_lo = 0, frame_hi = 0;            // packed-buffer range (multiples of 8 frames)
     JobRange eq, split, chain, wf, mb_chunks, kw, gain, lim;   // of the job table of the same name
+    JobRange meter_kw, meter_peak, meter_tracks;   // the output meter's tables (tracks with AME_F_MEASURE_OUTPUT only)
     int64_t seg_lo = 0, seg_hi = 0;
     int slot = 0;                                  // workspace slot (and stream) this wave runs in
     bool limiter = false;                          // a track of the wave has the limiter stage
@@ -146,6 +147,9 @@ struct Layout {
     int split_tile = 0, kw_tile_sb = 0;
     int lim_keep = 2;                       // queue entries a recorded limiter state holds: look-ahead frames + 2
     bool any_limiter = false, any_tp = false;
+    bool any_meter = false;                 // a track carries AME_F_MEASURE_OUTPUT
+    std::vector<TrackDev> meter_tdev;       // tdev with sb_offset into the meter's own sub-block energies (flagged tracks)
+    int64_t meter_sb_total = 0;             // sub-blocks of the flagged tracks
 };
 
 // The tables a plan uploads once.  Every job table is ordered by track, hence contiguous per wave.
@@ -158,6 +162,11 @@ struct JobTables {
     std::vector<KwJob> kw;
     std::vector<GainJob> gain, lim;         // limiter tiles: the same (begin, end, track) records, shorter tiles
     std::vector<AttEntry> att;              // 32769 entries per distinct compressor band
+    // output meter, flagged tracks only: K-weighting tiles (kw_tile_sb sub-blocks, as kw), peak tiles (the gain tiles)
+    // and the list of flagged tracks
+    std::vector<KwJob> meter_kw;
+    std::vector<GainJob> meter_peak;
+    std::vector<int32_t> meter_tracks;
 };
 
 struct DeviceShape {
@@ -284,6 +293,9 @@ inline int validate(const ame_track_params &t, int idx, std::string &err) {
             return layout_fail(err, AME_E_INVALID, "track %d: bad limiter parameters (look-ahead %d frames, release %d frames)", idx,
                                t.lim_frames, t.lim_release_frames);
     }
+    if ((t.flags & AME_F_MEASURE_OUTPUT) && t.halo_frames)
+        return layout_fail(err, AME_E_UNSUPPORTED, "track %d: the output meter measures a whole track and cannot run on a time "
+                                                   "shard; measure the gathered output instead", idx);
     for (int s = 0; s < 4; ++s) {
         const int k = t.eq[s].kind;
         const bool shelf = (s == 0 || s == 3);
@@ -372,6 +384,14 @@ inline int build_layout(const ame_track_params *tracks, int n_tracks, const ame_
         lay.any_limiter = lay.any_limiter || (tp.flags & AME_F_LIMITER);
         if (tp.flags & AME_F_LIMITER) lay.lim_keep = std::max(lay.lim_keep, tp.lim_frames + 2);
         lay.any_tp = lay.any_tp || (tp.flags & AME_F_TRUE_PEAK);
+        lay.any_meter = lay.any_meter || (tp.flags & AME_F_MEASURE_OUTPUT);
+    }
+    if (lay.any_meter) {
+        lay.meter_tdev = lay.tdev;
+        for (int t = 0; t < n_tracks; ++t) {
+            lay.meter_tdev[t].sb_offset = lay.meter_sb_total;
+            if (lay.tracks[t].flags & AME_F_MEASURE_OUTPUT) lay.meter_sb_total += lay.tdev[t].n_sb;
+        }
     }
     for (size_t i = 1; i < spans.size(); ++i)
         if (spans[i].first < align_up(spans[i - 1].second, 8))
@@ -632,6 +652,20 @@ inline int build_layout(const ame_track_params *tracks, int n_tracks, const ame_
             wv.limiter = wv.limiter || (lay.tracks[t].flags & AME_F_LIMITER);
             wv.true_peak = wv.true_peak || (lay.tracks[t].flags & AME_F_TRUE_PEAK);
         }
+        // the output meter: the same K-weighting and gain tiles as the input side, for the flagged tracks only
+        wv.meter_kw.lo = (int)jobs.meter_kw.size(); wv.meter_peak.lo = (int)jobs.meter_peak.size();
+        wv.meter_tracks.lo = (int)jobs.meter_tracks.size();
+        for (int t = wv.track_lo; t < wv.track_hi; ++t) {
+            const ame_track_params &tp = lay.tracks[t];
+            if (!(tp.flags & AME_F_MEASURE_OUTPUT)) continue;
+            jobs.meter_tracks.push_back(t);
+            for (int sb = 0; sb < lay.tdev[t].n_sb; sb += lay.kw_tile_sb)
+                jobs.meter_kw.push_back(KwJob{t, sb, std::min(sb + lay.kw_tile_sb, lay.tdev[t].n_sb), 0});
+            for (int64_t b = 0; b < tp.n_frames; b += kGainTile)
+                jobs.meter_peak.push_back(GainJob{tp.offset_frames + b, tp.offset_frames + std::min<int64_t>(b + kGainTile, tp.n_frames), t, 0});
+        }
+        wv.meter_kw.n = (int)jobs.meter_kw.size() - wv.meter_kw.lo; wv.meter_peak.n = (int)jobs.meter_peak.size() - wv.meter_peak.lo;
+        wv.meter_tracks.n = (int)jobs.meter_tracks.size() - wv.meter_tracks.lo;
         lay.slot_lim_jobs = std::max(lay.slot_lim_jobs, wv.lim.n);
         lay.slot_tiles = std::max(lay.slot_tiles, wv.wf.n);
         lay.slot_chains = std::max(lay.slot_chains, wv.chain.n);

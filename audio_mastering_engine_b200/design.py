@@ -256,5 +256,7 @@ def track_params(settings, fs, n_frames, offset_frames=0, chunk_seconds=30, lut_
         p.lim_thr_i = thr
     if settings.get("true_peak"):
         flags |= L.AME_F_TRUE_PEAK
+    if settings.get("measure_output"):                    # EBU R128 meter of the final output (ame_loudness)
+        flags |= L.AME_F_MEASURE_OUTPUT
     p.flags = flags
     return p

@@ -6,6 +6,7 @@ Public surface (same names / argument meaning / error behaviour as audio_masteri
   process_audio_with_ffmpeg_pipeline(settings, status_cb, progress_cb) -> path :171-226
 plus the in-memory API used by tests and benchmarks:
   master(samples, fs, settings) -> (int16[N,2], info)
+  measure_loudness(samples, fs) -> EBU R128 report of tracks that are not mastered
   MasterPlan - a reusable batch plan (packed layout, coefficients, device workspace).
 There is no CPU fallback: without libame.so or without a CUDA device these raise.
 """
@@ -29,6 +30,26 @@ log = logging.getLogger("audio_mastering_engine_b200")
 
 def _align8(n):
     return (int(n) + 7) // 8 * 8
+
+
+def _loudness_dict(r):
+    """One ame_loudness as a dict; tp is the true peak in dBTP."""
+    return dict(integrated=r.integrated, thresh=r.thresh, lra=r.lra, true_peak=r.true_peak,
+                tp=20.0 * math.log10(r.true_peak) if r.true_peak > 0 else -math.inf, sample_peak=int(r.sample_peak),
+                n_blocks=int(r.n_blocks), max_momentary=r.max_momentary, max_short_term=r.max_short_term)
+
+
+# the names a meter reading goes by in a mastering report (loudnorm's second-pass output_*) and in measure_loudness()
+OUTPUT_KEYS = dict(integrated="output_i", tp="output_tp", lra="output_lra", thresh="output_thresh",
+                   true_peak="output_true_peak", sample_peak="output_sample_peak", n_blocks="output_n_blocks",
+                   max_momentary="output_max_momentary", max_short_term="output_max_short_term")
+INPUT_KEYS = dict(integrated="input_i", tp="input_tp", lra="input_lra", thresh="input_thresh", true_peak="true_peak",
+                  sample_peak="sample_peak", n_blocks="n_blocks", max_momentary="max_momentary", max_short_term="max_short_term")
+
+
+def output_report(m):
+    """A meter reading (MasterPlan.output_loudness / measure_loudness entry) under the output_* keys of results()."""
+    return {OUTPUT_KEYS[k]: v for k, v in m.items()}
 
 
 class MasterPlan:
@@ -79,6 +100,8 @@ class MasterPlan:
                 luts[idx] = design.warm_lut(ac)
             L.check(self.lib.ame_plan_set_warm_luts(h, luts.ctypes.data_as(C.c_void_p), len(lut_index)))
         self._results = (L.TrackResult * n)()
+        # the output meter: tracks whose settings have "measure_output"
+        self._loudness = (L.Loudness * n)() if any(arr[i].flags & L.AME_F_MEASURE_OUTPUT for i in range(n)) else None
 
     # -- lifetime -----------------------------------------------------------------------------
     def close(self):
@@ -108,9 +131,12 @@ class MasterPlan:
     def results(self):
         """Per-track loudness report: the numbers ffmpeg's loudnorm prints as JSON (audio_mastering_engine.py:229-237),
         plus whether real ffmpeg would have stayed in LINEAR mode (static gain) - this build always applies the
-        static gain (DESIGN.md, deviation D3)."""
+        static gain (DESIGN.md, deviation D3).  Tracks with settings["measure_output"] also carry loudnorm's output_*
+        keys.  Both sides are those of the last call that fetched results (master_host, or master_device /
+        normalize_device with fetch_results=True); after a call with fetch_results=False, output_loudness() reads that
+        call's meter."""
         out = []
-        for r, s in zip(self._results, self.settings):
+        for k, (r, s) in enumerate(zip(self._results, self.settings)):
             d = dict(input_i=r.input_i, measured_i_2dp=r.measured_i_2dp, gain=r.gain,
                      rel_threshold_energy=r.rel_threshold, n_blocks=int(r.n_blocks),
                      normalized=bool(r.normalized), sample_peak=int(r.sample_peak),
@@ -123,8 +149,30 @@ class MasterPlan:
                 offset = float(s.get("lufs")) - r.measured_i_2dp
                 d["target_offset"] = offset
                 d["linear_mode_ok"] = bool(d["input_tp"] + offset <= -1.5 and r.input_lra <= 11.0)   # TP=-1.5:LRA=11 (:229)
+            if self._loudness is not None and self._loudness[k].measured:
+                d.update(output_report(_loudness_dict(self._loudness[k])))    # loudnorm's second-pass output_*
             out.append(d)
         return out
+
+    def _fetch_loudness(self, stream=None):
+        if self._loudness is not None:
+            L.check(self.lib.ame_plan_output_loudness(self.handle, self._loudness, C.c_void_p(stream or 0)))
+
+    def output_loudness(self, stream=None):
+        """EBU R128 meter of the final output of the last master_device / master_host / normalize_device call: per track
+        a dict (integrated, thresh, lra, true_peak, tp, sample_peak, n_blocks, max_momentary, max_short_term), or None
+        for a track without settings["measure_output"] or before any call.  `stream` must be ordered after that call."""
+        if self._loudness is None:
+            return [None] * self.n_tracks
+        self._fetch_loudness(stream)
+        return [_loudness_dict(r) if r.measured else None for r in self._loudness]
+
+    def measure_loudness(self, d_buf, stream=None):
+        """The stand-alone meter: the same report for the flagged tracks of any CUDA int16 buffer in this plan's packed
+        layout (synchronous).  Raises when no track has settings["measure_output"]."""
+        res = (L.Loudness * self.n_tracks)()
+        L.check(self.lib.ame_measure_loudness(self.handle, self._ptr(d_buf), res, C.c_void_p(stream or 0)))
+        return [_loudness_dict(r) if r.measured else None for r in res]
 
     @property
     def launch_count(self):
@@ -168,11 +216,14 @@ class MasterPlan:
         """d_in / d_out: CUDA int16 tensors (or raw device pointers) of total_frames*2 samples."""
         res = self._results if fetch_results else None
         L.check(self.lib.ame_master_device(self.handle, self._ptr(d_in), self._ptr(d_out), res, C.c_void_p(stream or 0)))
+        if fetch_results:
+            self._fetch_loudness(stream)
         return self.results() if fetch_results else None
 
     def master_host(self, h_in, h_out):
         """h_in / h_out: host int16 arrays (numpy, or pinned torch CPU tensors) in the packed layout."""
         L.check(self.lib.ame_master_host(self.handle, self._ptr(h_in), self._ptr(h_out), self._results))
+        self._fetch_loudness()                             # master_host returns synchronised, meter included
         return self.results()
 
     def measure_device(self, d_in, d_hist, stream=None):
@@ -181,6 +232,8 @@ class MasterPlan:
     def normalize_device(self, d_hist, d_out, stream=None, fetch_results=True):
         res = self._results if fetch_results else None
         L.check(self.lib.ame_normalize_device(self.handle, self._ptr(d_hist), self._ptr(d_out), res, C.c_void_p(stream or 0)))
+        if fetch_results:
+            self._fetch_loudness(stream)
         return self.results() if fetch_results else None
 
     def set_timing(self, enable=True):
@@ -298,6 +351,46 @@ def master(samples, fs, settings, device=0, chunk_seconds=30, **plan_opts):
     finally:
         plan.close()
     return (outs[0], infos[0]) if single else (outs, infos)
+
+
+def _meter(tracks, fs, device=0):
+    """Stand-alone EBU R128 meter of int16 tracks (numpy arrays or torch tensors, [N,2] or mono [N]) on `device`: a plan
+    whose tracks carry only the meter flag, the tracks uploaded into its packed layout.  One dict per track (see
+    MasterPlan.output_loudness)."""
+    import torch
+    dev = torch.device("cuda", device)
+    ts = []
+    for x in tracks:
+        x = x if isinstance(x, torch.Tensor) else torch.from_numpy(_as_stereo_pcm(x))
+        if x.dtype != torch.int16:
+            raise TypeError("samples must be int16")
+        if x.ndim == 1:
+            x = torch.stack([x, x], dim=1)
+        if x.ndim != 2 or x.shape[1] != 2:
+            raise ValueError("samples must have shape [N] or [N,2]")
+        ts.append(x)
+    n = len(ts)
+    fs_list = [fs] * n if np.isscalar(fs) else list(fs)
+    plan = MasterPlan([t.shape[0] for t in ts], fs_list, {"lufs": None, "measure_output": True}, device=device, chunk_seconds=None)
+    try:
+        buf = torch.zeros((plan.total_frames, 2), dtype=torch.int16, device=dev)
+        for t, off in zip(ts, plan.offsets):
+            buf[off:off + t.shape[0]] = t.to(dev)
+        with torch.cuda.device(dev):
+            return plan.measure_loudness(buf, stream=torch.cuda.current_stream(dev).cuda_stream)
+    finally:
+        plan.close()
+
+
+def measure_loudness(samples, fs, device=0):
+    """EBU R128 / BS.1770 meter on the GPU without mastering anything: integrated loudness (input_i, LUFS), relative gate
+    (input_thresh), loudness range (input_lra), true peak (true_peak linear, input_tp dBTP; BS.1770 Annex 2 below 192 kHz),
+    sample_peak, n_blocks and the maxima of the momentary and short-term loudness.  samples: int16[N,2] (or [N] mono,
+    numpy or torch), or a list of such tracks (fs may then be a list too).  Returns a dict, or a list of dicts."""
+    single = not isinstance(samples, (list, tuple))
+    ms = _meter([samples] if single else list(samples), fs, device)
+    out = [{INPUT_KEYS[k]: v for k, v in m.items()} for m in ms]
+    return out[0] if single else out
 
 
 LIMITER_KEYS = ("limiter", "limiter_limit", "limiter_attack", "limiter_release")
@@ -438,6 +531,11 @@ def process_audio_with_ffmpeg_pipeline(settings, status_callback, progress_callb
     status_callback("Applying final limiting and exporting...")
     progress_callback(num_chunks + 3, total_steps)
     write_wav(output_file, out, fs)
+    if settings.get("measure_output"):
+        msg = (f"Final loudness: {info['output_i']:.2f} LUFS integrated, {info['output_tp']:.2f} dBTP true peak, "
+               f"LRA {info['output_lra']:.1f} LU")
+        log.info(msg)
+        status_callback(msg)
     progress_callback(total_steps, total_steps)
     log.info("Finished GPU pipeline, exported to %s", output_file)
     return output_file

@@ -174,10 +174,18 @@ def time_sharded_step(sh, spans, group=None):
 
 
 def _shard_settings(settings):
-    """What the shards run: everything but the limiter, which is one sequential machine over the whole track."""
+    """What the shards run: everything but the limiter, which is one sequential machine over the whole track, and the
+    output meter, which measures the whole track (a shard's output is not the track's output)."""
     st = dict(settings)
     st["limiter"] = False
+    st.pop("measure_output", None)
     return st
+
+
+def _with_output_report(info, full, fs, device):
+    """info + the EBU R128 meter of the joined (and limited) track `full` under the output_* keys."""
+    from .engine import _meter, output_report
+    return dict(info or {}, **output_report(_meter([full], fs, device)[0]))
 
 
 def _gather_spans(out, spans, group, dst=0):
@@ -214,7 +222,11 @@ def master_time_sharded(track, fs, settings, group=None, device=None, chunk_seco
 
     With settings["limiter"] (the reference's alimiter, :223) the normalised spans are gathered on rank 0, which runs
     the limiter over the whole track (engine.limit_device - parallel in time on ONE GPU, but not across shards) and
-    returns (0, the whole limited track, info); the other ranks return (span_begin, an empty array, info)."""
+    returns (0, the whole limited track, info); the other ranks return (span_begin, an empty array, info).
+
+    With settings["measure_output"] the spans are gathered on rank 0 too, which meters the joined (and limited) track
+    and adds the report to its info under the output_* keys of MasterPlan.results(); what each rank returns is as
+    without it."""
     import torch
     import torch.distributed as dist
     from .engine import limit_device
@@ -225,14 +237,21 @@ def master_time_sharded(track, fs, settings, group=None, device=None, chunk_seco
     span = track[spans[rank][0]:spans[rank][1]]
     sh.load(span if hasattr(span, "device") else np.ascontiguousarray(span))
     out, info, _ = time_sharded_step(sh, spans, group)
+    measure = bool(settings.get("measure_output"))
     if settings.get("limiter"):
         full = _gather_spans(out, spans, group)
         sh.close()
         if full is None:
             return spans[rank][0], np.zeros((0, 2), dtype=np.int16), info
-        return 0, limit_device(full, fs, settings, device).cpu().numpy(), info
+        full = limit_device(full, fs, settings, device)
+        if measure:
+            info = _with_output_report(info, full, fs, device)
+        return 0, full.cpu().numpy(), info
+    full = _gather_spans(out, spans, group) if measure else None
     res = out.cpu().numpy()
     sh.close()
+    if full is not None:
+        info = _with_output_report(info, full, fs, device)
     return spans[rank][0], res, info
 
 
@@ -267,4 +286,6 @@ def master_time_sharded_local(track, fs, settings, world, device=0, chunk_second
     full = torch.cat(outs, dim=0)
     if settings.get("limiter"):
         full = limit_device(full, fs, settings, device)
+    if settings.get("measure_output"):
+        info = _with_output_report(info, full, fs, device)
     return full.cpu().numpy(), info

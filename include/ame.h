@@ -48,6 +48,8 @@ typedef enum {
 #define AME_F_NORMALIZE 8u  /* settings["lufs"] is not None    (:216) */
 #define AME_F_LIMITER   16u /* the final ffmpeg alimiter       (:223); not for time shards (global sequential state) */
 #define AME_F_TRUE_PEAK 32u /* also measure the BS.1770 Annex 2 true peak of the pre-normalisation signal */
+#define AME_F_MEASURE_OUTPUT 64u /* meter the track's final output (ame_loudness); not for time shards (a shard's output is
+                                    not the track's output) */
 
 /* EQ stage kinds (apply_shelf_filter :283-289, apply_peak_filter :290-298) */
 #define AME_EQ_BYPASS      0  /* gain == 0: stage returns its input untouched */
@@ -127,6 +129,21 @@ typedef struct {
                                 the sample peak / 32768 when AME_F_TRUE_PEAK is not set or fs >= 192 kHz */
 } ame_track_result;
 
+/* EBU R128 meter of one track (AME_F_MEASURE_OUTPUT): what ffmpeg's loudnorm prints as output_* in its second pass, plus
+ * the maxima of the ungated momentary (400 ms) and short-term (3 s) loudness, both taken every 100 ms.  integrated,
+ * thresh, lra, n_blocks, sample_peak and true_peak are computed exactly as the input side of ame_track_result is. */
+typedef struct {
+    double integrated;      /* LUFS (ebur128 gated); -inf when no block passes the gate */
+    double thresh;          /* relative gate threshold, LUFS; -70 when no block passes the absolute gate */
+    double lra;             /* loudness range, LU */
+    double true_peak;       /* linear; BS.1770 Annex 2 (4x below 96 kHz, 2x below 192 kHz), else sample peak / 32768 */
+    double max_momentary;   /* LUFS; -inf when the track has no complete 400 ms window */
+    double max_short_term;  /* LUFS; -inf when the track has no complete 3 s window */
+    int64_t n_blocks;       /* 400 ms blocks above the absolute gate */
+    int32_t sample_peak;    /* max |s16| over every frame of the track */
+    int32_t measured;       /* 1 when this entry holds a measurement */
+} ame_loudness;
+
 typedef struct {
     int32_t eq_tile_frames;      /* 0 = choose from the batch size */
     int32_t xover_tile_frames;   /* 0 = auto */
@@ -155,6 +172,7 @@ int ame_abi_version(void);
 size_t ame_sizeof_track_params(void);
 size_t ame_sizeof_track_result(void);
 size_t ame_sizeof_plan_options(void);
+size_t ame_sizeof_loudness(void);
 const char *ame_last_error(void);             /* thread-local text of the last failure */
 int ame_device_count(int *count);
 /* plan workspaces are taken from a per-device memory pool that keeps the memory of destroyed plans for the next one
@@ -170,7 +188,8 @@ void ame_plan_destroy(ame_plan *plan);
 int ame_plan_set_warm_luts(ame_plan *plan, const float *luts, int32_t n_luts);
 int64_t ame_plan_total_frames(const ame_plan *plan);     /* padded length of the packed buffers */
 size_t ame_plan_workspace_bytes(const ame_plan *plan);
-int64_t ame_plan_launch_count(const ame_plan *plan);      /* kernels launched by the last call */
+int64_t ame_plan_launch_count(const ame_plan *plan);      /* kernels launched by the last ame_master_* / ame_measure_device /
+                                                             ame_measure_loudness call (the meter's launches included) */
 int32_t ame_plan_wave_count(const ame_plan *plan);
 int32_t ame_plan_slot_count(const ame_plan *plan);
 /* statistics of the compressor recurrence of the last call (benchmarks): chains, flagged steps in total and in the
@@ -208,6 +227,17 @@ int ame_master_device(ame_plan *plan, const int16_t *d_in, int16_t *d_out,
 /* same with HOST buffers (pinned or pageable): H2D, the chain, D2H - pipelined over the plan's waves -
  * synchronised on return. */
 int ame_master_host(ame_plan *plan, const int16_t *h_in, int16_t *h_out, ame_track_result *results);
+
+/* EBU R128 meter.  When tracks carry AME_F_MEASURE_OUTPUT, ame_master_device, ame_master_host and ame_normalize_device
+ * also meter the FINAL output of those tracks (after the gain, and after the limiter when the track has one), on the
+ * streams the call runs on; ame_plan_output_loudness copies those results on `stream` (which must be ordered after the
+ * call) and synchronises it.  Before any such call every entry has measured = 0.  out: HOST array of n_tracks entries;
+ * tracks without the flag get measured = 0.  The ame_stage_* entry points do not meter. */
+int ame_plan_output_loudness(ame_plan *plan, ame_loudness *out, void *stream);
+/* stand-alone meter: every track that carries AME_F_MEASURE_OUTPUT, read from d_buf (any DEVICE buffer in the plan's
+ * packed layout; the other flags of the track do not matter), on `stream`.  out (may be NULL) is filled synchronously.
+ * AME_E_INVALID when no track carries the flag.  Does not touch what ame_plan_output_loudness reports. */
+int ame_measure_loudness(ame_plan *plan, const int16_t *d_buf, ame_loudness *out, void *stream);
 
 /* two-phase form for tracks that are time-sharded across GPUs: phase 1 stops after the gating
  * histograms (d_hist: DEVICE int64[n_tracks][1000], caller-owned so it can be all-reduced with
