@@ -84,6 +84,7 @@ SYMBOLS = {
     "ame_plan_wave_count": (C.c_int32, [C.c_void_p]),
     "ame_plan_slot_count": (C.c_int32, [C.c_void_p]),
     "ame_plan_limiter_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "ame_plan_set_limiter_guess": (C.c_int, [C.c_void_p, C.c_int32]),
     "ame_plan_chain_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
                                       C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
     "ame_plan_set_timing": (C.c_int, [C.c_void_p, C.c_int]),

@@ -157,6 +157,7 @@ struct ame_plan : Layout {
     int *d_peak = nullptr;
     unsigned *d_tp = nullptr;               // per track: float bits of the oversampled peak (k_true_peak)
     int *d_lim_stats = nullptr;             // open tiles after the limiter's round 0 / 1 / 2, accumulated
+    int lim_guess = -1;                     // frames of the limiter's round-0 guess; -1 = 2 G (ame_plan_set_limiter_guess)
     ame_track_result *d_results = nullptr;
     // output meter (tracks with AME_F_MEASURE_OUTPUT; none of it exists without such a track)
     KwJob *d_meter_kw = nullptr;
@@ -387,10 +388,10 @@ int run_apply(ame_plan *p, const Wave &w, const int16_t *d_pre, int16_t *d_out, 
         const size_t smem = lim_smem_bytes(cap);
         for (int round = 0; round <= kLimRounds; ++round) {
             if (round == 0) {                         // the elementwise tiles, 256 threads each
-                k_limiter<<<w.lim.n, 256, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, 0, cap);
+                k_limiter<<<w.lim.n, 256, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, 0, cap, p->lim_guess);
                 LAUNCH_CHECK(p);
             }
-            k_limiter<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, round, cap);
+            k_limiter<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, round, cap, p->lim_guess);
             LAUNCH_CHECK(p);
             k_lim_verify<<<(w.lim.n + 3) / 4, 128, 0, s>>>(gj, w.lim.n, p->d_tracks, b.lim_in, b.lim_out, b.lim_need,
                                                              p->d_lim_stats + round);
@@ -717,6 +718,13 @@ int ame_plan_limiter_stats(ame_plan *p, int64_t *open_tiles) {
     CU(cudaMemcpy(h, p->d_lim_stats, sizeof h, cudaMemcpyDeviceToHost));
     CU(cudaMemset(p->d_lim_stats, 0, sizeof h));
     for (int i = 0; i < 3; ++i) open_tiles[i] = h[i];
+    return AME_OK;
+}
+
+int ame_plan_set_limiter_guess(ame_plan *p, int32_t frames) {
+    if (!p) return fail(AME_E_INVALID, "NULL plan");
+    if (frames < -1) return fail(AME_E_INVALID, "limiter guess of %d frames (-1 = the default 2 G, or >= 0)", frames);
+    p->lim_guess = frames;
     return AME_OK;
 }
 

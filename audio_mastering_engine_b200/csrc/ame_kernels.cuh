@@ -1457,11 +1457,12 @@ __device__ __forceinline__ LimCtx lim_ctx(const ame_track_params *tp, const int1
 }
 
 // round 0: every tile (elementwise tiles by all threads, the others by warp 0 from the initial state or from a guess);
-// round >= 1: the tiles k_lim_verify left open, from their predecessor's recorded end state
+// round >= 1: the tiles k_lim_verify left open, from their predecessor's recorded end state.
+// guess: frames the round-0 guess runs over in front of its tile; -1 = 2 G (ame_plan_set_limiter_guess)
 __global__ void __launch_bounds__(256)
 k_limiter(const GainJob *__restrict__ jobs, int n_jobs, const long long *__restrict__ lim_last,
           const ame_track_params *__restrict__ tracks, const int16_t *__restrict__ norm, int16_t *__restrict__ out,
-          LimStore IN, LimStore OUT, int *__restrict__ need, int round, int cap) {
+          LimStore IN, LimStore OUT, int *__restrict__ need, int round, int cap, int guess) {
     // round 0 is launched twice: 256 threads per tile for the elementwise tiles (the others leave at once) and ONE warp
     // per tile for the sequential ones (so that a few thousand of them are resident at a time)
     extern __shared__ __align__(16) unsigned char lim_raw[];
@@ -1488,7 +1489,7 @@ k_limiter(const GainJob *__restrict__ jobs, int n_jobs, const long long *__restr
         lim_reset(r, sm, lane);
         int exact = 1;
         if (!t.quiet_start) {                                         // guess: the machine over the 2 G frames in front
-            const int64_t ws = max(c.t_begin, job.begin - 2 * t.G);
+            const int64_t ws = max(c.t_begin, job.begin - (guess < 0 ? 2 * t.G : (int64_t)guess));
             exact = ws == c.t_begin;                                  // from the track start it is no guess
             lim_run(c, r, sm, ws, job.begin, false, lane);
         }

@@ -196,6 +196,11 @@ class MasterPlan:
         L.check(self.lib.ame_plan_limiter_stats(self.handle, v))
         return [int(x) for x in v]
 
+    def set_limiter_guess(self, frames=-1):
+        """Test knob: frames the limiter's round-0 guess of a tile's start state runs over (-1 = the default 2 G;
+        0 = no guess, a wrong start on every clipping tile).  Changes how much repair work runs, never the output."""
+        L.check(self.lib.ame_plan_set_limiter_guess(self.handle, int(frames)))
+
     def chain_stats(self):
         """Compressor recurrence of the last call: chains, flagged steps (total, longest chain), passes (total, max)."""
         v = [C.c_int64() for _ in range(4)]

@@ -199,6 +199,13 @@ int32_t ame_plan_slot_count(const ame_plan *plan);
 int ame_plan_limiter_stats(ame_plan *plan, int64_t *open_tiles /* [3] */);
 int ame_plan_chain_stats(ame_plan *plan, int64_t *n_chains, int64_t *steps, int64_t *max_steps, int64_t *passes,
                          int32_t *max_passes);
+/* limiter, diagnostic / test knob: the round-0 guess of a tile's start state runs the machine from the initial state
+ * over `frames` frames in front of the tile (clipped at the track start; only a guess that reaches the track start
+ * counts as exact).  -1 (the default) = 2 G frames, G = look-ahead + release + 8; 0 = every tile that does not start
+ * in the initial state starts from it, a wrong guess on every such tile of a clipping track.  Shorter windows give
+ * wrong guesses and so run the repair rounds and the sequential fallback; the output is the same for every value.
+ * Applies to the following calls of the plan. */
+int ame_plan_set_limiter_guess(ame_plan *plan, int32_t frames);
 
 /* per-kernel device timing with CUDA events on the processing stream(s) (benchmarks): enable, run up to 64
  * ame_master_* / ame_measure_* calls, then read the summed milliseconds and launch counts per kernel (with
