@@ -386,7 +386,7 @@ k_band_split(const __grid_constant__ XoverCfg xc, const TileJob *__restrict__ jo
 //                                     low.overlay(mid).overlay(high) (:309).
 // pydub: rms_at(i) = audioop.rms(frames [max(i-look,0), i)) = (unsigned)sqrt(S / n) with S the exact integer
 // sum of squares and n = 2 * frames.  rms > thresh  <=>  rms >= thr_i  <=>  S >= thr_i^2 * n (integers), so
-// only flagged frames take the square root (S/n is never within 2^-41 of a perfect square unless equal,
+// only flagged frames take the square root (S/n is never within a relative 2^-43 of a perfect square unless equal,
 // hence the double-precision expression of audioop truncates to the exact integer root).
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ unsigned energy_of(uint32_t w) {          // l^2 + r^2 <= 2^31
@@ -406,9 +406,13 @@ __device__ __forceinline__ void load8(const uint32_t *__restrict__ p, int64_t id
     }
 }
 
-// floor(sqrt(s / n)) in exact integers, for s / n < 2^31 and n < 2^11: audioop.rms is (unsigned)sqrt(S / n) in double,
-// which truncates to exactly this (header comment above) - a float estimate is within 1 of it, two integer tests
-// settle it, and the double division + square root (~55 instructions on the FP64 pipe per flagged frame) go away.
+// floor(sqrt(s / n)) in exact integers, for s / n <= 2^30 (rms <= 32768) and n = 2 * window frames <= 8192 (look_frames
+// <= 4096 is validated; 384 kHz needs 3840): audioop.rms is (unsigned)sqrt(S / n) in double, which truncates to exactly
+// this (header comment above: S / n below a square k^2 stays below it by >= 1 / n, a relative 2^-43, far more than the
+// double division and root can lose).  The float estimate (float(s), __fdividef within 2 ulp, a rounded root) is within
+// 2^-20 relative, < 0.04 absolute, of the root, so truncation leaves it within 1; two integer tests settle it without
+// overflow ((2^15 + 1)^2 * 2^13 < 2^44), and the double division + square root (~55 FP64 instructions per flagged frame)
+// go away.
 __device__ __forceinline__ unsigned isqrt_ratio(unsigned long long s, unsigned n) {
     unsigned r = (unsigned)__fsqrt_rn(__fdividef((float)s, (float)n));
     if ((unsigned long long)r * r * n > s) --r;

@@ -324,6 +324,11 @@ inline int validate(const ame_track_params &t, int idx, std::string &err) {
             if (!(c.thresh_rms >= 0) || !(c.attack_frames > 0) || !(c.release_frames > 0) || c.look_frames < 0 ||
                 c.look_frames > 4096)
                 return layout_fail(err, AME_E_INVALID, "track %d: bad compressor band %d", idx, b);
+            // ratio < 1 makes max_attenuation negative: k_att_chain orders attenuations by their bit patterns and shifts
+            // parked segments by whole ulps, which holds for non-negative operands only
+            if (!(c.coef >= 0))
+                return layout_fail(err, AME_E_UNSUPPORTED, "track %d: compressor band %d has a ratio below 1 (1 - 1/ratio = %g)",
+                                   idx, b, c.coef);
         }
     return AME_OK;
 }
