@@ -1059,7 +1059,8 @@ k_block_hist(const TrackDev *__restrict__ tdev, int track_lo, const double *__re
 }
 
 // ebur128_gated_loudness over a 400 ms block histogram, in ebur128.c's order (the sums are order-sensitive in the last
-// bit, and that bit can decide the '%.2f' the gain is made of): blocks above the absolute gate, the relative gate (as
+// bit, and that bit can decide the '%.2f' the gain is made of; products and sums rounded separately, as the C library
+// computes them - an FMA there moved the relative gate by one ulp): blocks above the absolute gate, the relative gate (as
 // energy and in LUFS; -70 when no block passes) and the gated loudness (-inf when no block passes the relative gate).
 // k_finalize and k_meter_finalize both walk with it.
 struct GateWalk { long long count, above; double rel, thresh, integrated; };
@@ -1067,7 +1068,7 @@ template <class H>
 __device__ __forceinline__ GateWalk gate_walk(const H *h) {
     GateWalk g{0, 0, 0.0, -70.0, -INFINITY};
     double rel = 0.0; long long count = 0;
-    for (int j = 0; j < 1000; ++j) { rel += (double)h[j] * c_hist_energy[j]; count += h[j]; }
+    for (int j = 0; j < 1000; ++j) { rel = __dadd_rn(rel, __dmul_rn((double)h[j], c_hist_energy[j])); count += h[j]; }
     g.count = count;
     if (count > 0) {
         rel /= (double)count;
@@ -1078,7 +1079,7 @@ __device__ __forceinline__ GateWalk gate_walk(const H *h) {
         if (rel < c_hist_bounds[0]) start = 0;
         else { start = hist_index(rel); if (rel > c_hist_energy[start]) ++start; }
         double gated = 0.0; long long above = 0;
-        for (int j = start; j < 1000; ++j) { gated += (double)h[j] * c_hist_energy[j]; above += h[j]; }
+        for (int j = start; j < 1000; ++j) { gated = __dadd_rn(gated, __dmul_rn((double)h[j], c_hist_energy[j])); above += h[j]; }
         g.above = above;
         if (above > 0) {
             gated /= (double)above;
@@ -1093,7 +1094,7 @@ __device__ __forceinline__ GateWalk gate_walk(const H *h) {
 template <class HS>
 __device__ __forceinline__ double lra_walk(const HS *hs) {
     long long n = 0; double power = 0.0;
-    for (int j = 0; j < 1000; ++j) { n += hs[j]; power += (double)hs[j] * c_hist_energy[j]; }
+    for (int j = 0; j < 1000; ++j) { n += hs[j]; power = __dadd_rn(power, __dmul_rn((double)hs[j], c_hist_energy[j])); }
     if (n > 0) {
         power /= (double)n;
         const double integ = 0.01 * power;           // MINUS_20DB
