@@ -108,7 +108,7 @@ enum { S_EQ = 0, S_SPLIT, S_FLAG, S_CHAIN, S_APPLY, S_KW, S_TAIL, S_HIST, S_FIN,
 
 // Per-wave workspace.  A plan has n_slots of them; wave w runs in slot w % n_slots on that slot's stream, so a slot is
 // recycled in stream order and a plan over many waves needs the intermediate buffers of only n_slots waves.
-struct Slot {
+struct Workspace {
     int16_t *pre = nullptr;      // pre-normalisation int16 of the wave (the signal the reference materialises at the concat)
     int16_t *bands = nullptr;    // 3 planes of mb_frames frames
     uint16_t *rms = nullptr;     // 3 planes: integer window rms of flagged frames, 0 elsewhere
@@ -121,6 +121,9 @@ struct Slot {
     long long *lim_last = nullptr;   // per k_apply_gain tile: last frame over the limiter's limit, or -1
     LimStore lim_in{}, lim_out{};    // per tile: the limiter state it started from / ended in
     int *lim_need = nullptr;         // per tile: its start is not its predecessor's end (yet)
+};
+
+struct Slot : Workspace {
     cudaStream_t stream = nullptr;
 };
 
@@ -183,20 +186,27 @@ struct ame_plan : Layout {
 
 namespace {
 
-inline bool t_on(const ame_plan *p) {
-    return p->timing && p->t_step >= 0 && p->t_step < kMaxTimedSteps && p->t_wave < kMaxTimedWaves;
+// after every kernel launch: a failed launch fails the call, a good one is counted (ame_plan_launch_count)
+int launched(ame_plan *p) {
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(AME_E_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
+    ++p->launches;
+    return AME_OK;
 }
-inline size_t t_slot(const ame_plan *p, int kernel) {
-    return ((size_t)p->t_step * kMaxTimedWaves + p->t_wave) * AME_N_KERNELS + kernel;
-}
-inline void t_begin(ame_plan *p, int kernel, cudaStream_t s) {
-    if (t_on(p)) cudaEventRecord(p->t_ev[t_slot(p, kernel) * 2], s);
-}
-inline void t_end(ame_plan *p, int kernel, cudaStream_t s) {
-    if (t_on(p)) {
-        cudaEventRecord(p->t_ev[t_slot(p, kernel) * 2 + 1], s);
-        p->t_used[t_slot(p, kernel)] = 1;
+
+// Runs `launches` (one stage's launches, each checked by launched()) between the two CUDA events of the stage's timing
+// slot; a stage that failed records no end, and its error names the stage.
+template <class F>
+int timed(ame_plan *p, int kernel, cudaStream_t s, F &&launches) {
+    const bool on = p->timing && p->t_step >= 0 && p->t_step < kMaxTimedSteps && p->t_wave < kMaxTimedWaves;
+    const size_t slot = ((size_t)p->t_step * kMaxTimedWaves + p->t_wave) * AME_N_KERNELS + kernel;
+    if (on) cudaEventRecord(p->t_ev[slot * 2], s);
+    if (int rc = launches()) return fail(rc, "%s stage: %s", kKernelNames[kernel], g_err.c_str());
+    if (on) {
+        cudaEventRecord(p->t_ev[slot * 2 + 1], s);
+        p->t_used[slot] = 1;
     }
+    return AME_OK;
 }
 
 // The one allocator of a plan's device memory: it records every pointer, and ame_plan_destroy frees what it recorded.
@@ -226,13 +236,6 @@ int upload(ame_plan *p, T **dptr, const std::vector<T> &v) {
     return AME_OK;
 }
 
-#define LAUNCH_CHECK(p)                                                                            \
-    do {                                                                                           \
-        cudaError_t e_ = cudaGetLastError();                                                       \
-        if (e_ != cudaSuccess) return fail(AME_E_CUDA, "kernel launch failed: %s (%s:%d)", cudaGetErrorString(e_), __FILE__, __LINE__); \
-        ++(p)->launches;                                                                           \
-    } while (0)
-
 int check_warmth(const ame_plan *p) {
     for (int t = 0; t < p->n_tracks; ++t)
         if (p->tracks[t].flags & AME_F_WARMTH) {
@@ -242,60 +245,63 @@ int check_warmth(const ame_plan *p) {
     return AME_OK;
 }
 
+// the start of a call that runs the whole chain or its first phase: a new launch count and a new timed step
+int begin_call(ame_plan *p) {
+    if (int rc = check_warmth(p)) return rc;
+    p->launches = 0;
+    if (p->timing) ++p->t_step;
+    return AME_OK;
+}
+
 // ---- stage launches over one wave ------------------------------------------------------------------
-// `pre` is addressed with ABSOLUTE packed-buffer frame indices everywhere: for a slot the pointer handed in is
-// slot.pre - 2 * wave.frame_lo (never dereferenced outside the wave's own range).
-struct Bufs {
+// Every buffer the stages of one wave use: its slot's workspace and the caller's buffers.  `pre` and `norm` are
+// addressed with ABSOLUTE packed-buffer frame indices everywhere: for a slot they point at slot.pre - 2 * wave.frame_lo
+// (never dereferenced outside the wave's own range).  A stage entry point may put a read-only caller buffer (const_cast)
+// only where its stages do not write.
+struct Bufs : Workspace {
     const int16_t *in = nullptr;
-    int16_t *pre = nullptr, *bands = nullptr, *out = nullptr;
-    uint16_t *rms = nullptr, *list = nullptr;
-    int *tile_cnt = nullptr, *n_flagged = nullptr;
-    GrpRec *grp = nullptr;
-    double *att = nullptr;
+    int16_t *out = nullptr;
     int64_t *hist = nullptr;
-    int16_t *norm = nullptr;
-    long long *lim_last = nullptr;
-    LimStore lim_in{}, lim_out{};
-    int *lim_need = nullptr;
 };
 
-Bufs slot_bufs(ame_plan *p, const Wave &w, const int16_t *d_in, int16_t *d_out) {
-    const Slot &sl = p->slots[w.slot];
+// The buffers of wave w, whose launches are timed as wave w's from here on.
+Bufs start_wave(ame_plan *p, int w, const int16_t *d_in = nullptr, int16_t *d_out = nullptr) {
+    const Wave &wv = p->waves[w];
+    p->t_wave = std::min(w, kMaxTimedWaves - 1);
     Bufs b;
-    b.in = d_in; b.out = d_out;
-    b.pre = sl.pre - 2 * w.frame_lo;
-    b.bands = sl.bands; b.rms = sl.rms; b.list = sl.list; b.tile_cnt = sl.tile_cnt; b.n_flagged = sl.n_flagged;
-    b.grp = sl.grp; b.att = sl.att;
-    b.norm = sl.norm ? sl.norm - 2 * w.frame_lo : nullptr;
-    b.lim_last = sl.lim_last; b.lim_in = sl.lim_in; b.lim_out = sl.lim_out; b.lim_need = sl.lim_need;
+    static_cast<Workspace &>(b) = p->slots[wv.slot];
+    b.pre -= 2 * wv.frame_lo;
+    if (b.norm) b.norm -= 2 * wv.frame_lo;
+    b.in = d_in;
+    b.out = d_out;
     b.hist = (int64_t *)p->d_hist;
     return b;
 }
 
-int run_eq(ame_plan *p, const Wave &w, const int16_t *d_in, int16_t *d_pre, cudaStream_t s) {
+// k_eq, or k_eq_f32 for the precision experiment, and the block size it is launched with
+struct EqKernel {
+    decltype(&k_eq) fn;
+    int block;
+};
+EqKernel eq_kernel(const ame_plan *p) { return p->precision == 1 ? EqKernel{k_eq_f32, 128} : EqKernel{k_eq, kEqBlock}; }
+
+int run_eq(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     if (!w.eq.n) return AME_OK;
-    t_begin(p, S_EQ, s);
-    if (p->precision == 1)
-        k_eq_f32<<<(w.eq.n + 127) / 128, 128, 0, s>>>(p->d_eq_jobs + w.eq.lo, w.eq.n, p->d_tracks, p->d_luts, d_in, d_pre);
-    else
-        k_eq<<<(w.eq.n + kEqBlock - 1) / kEqBlock, kEqBlock, 0, s>>>(p->d_eq_jobs + w.eq.lo, w.eq.n, p->d_tracks, p->d_luts, d_in, d_pre);
-    LAUNCH_CHECK(p);
-    t_end(p, S_EQ, s);
-    return AME_OK;
+    const EqKernel k = eq_kernel(p);
+    return timed(p, S_EQ, s, [&] {
+        k.fn<<<(w.eq.n + k.block - 1) / k.block, k.block, 0, s>>>(p->d_eq_jobs + w.eq.lo, w.eq.n, p->d_tracks, p->d_luts, b.in, b.pre);
+        return launched(p);
+    });
 }
 
-int run_split(ame_plan *p, const Wave &w, const int16_t *d_pre, int16_t *d_bands, cudaStream_t s) {
+int run_split(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     if (!w.split.n) return AME_OK;
-    t_begin(p, S_SPLIT, s);
-    if (w.xover_uni)
-        k_band_split<true><<<(w.split.n + 127) / 128, 128, 0, s>>>(w.xover, p->d_split_jobs + w.split.lo, w.split.n, p->d_tracks, p->d_mb_delta,
-                                                                   d_pre, d_bands, p->mb_frames);
-    else
-        k_band_split<false><<<(w.split.n + 127) / 128, 128, 0, s>>>(w.xover, p->d_split_jobs + w.split.lo, w.split.n, p->d_tracks, p->d_mb_delta,
-                                                                    d_pre, d_bands, p->mb_frames);
-    LAUNCH_CHECK(p);
-    t_end(p, S_SPLIT, s);
-    return AME_OK;
+    auto *k = w.xover_uni ? k_band_split<true> : k_band_split<false>;
+    return timed(p, S_SPLIT, s, [&] {
+        k<<<(w.split.n + 127) / 128, 128, 0, s>>>(w.xover, p->d_split_jobs + w.split.lo, w.split.n, p->d_tracks, p->d_mb_delta,
+                                                  b.pre, b.bands, p->mb_frames);
+        return launched(p);
+    });
 }
 
 // Lanes (time segments) per chain of k_att_chain.  More lanes = shorter segments = cheaper passes but more of them once
@@ -312,75 +318,77 @@ int chain_lanes(const ame_plan *p, int n_chains) {
 
 int run_compress(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     if (!w.chain.n) return AME_OK;
-    t_begin(p, S_FLAG, s);
     int *tile_base = b.tile_cnt + std::max(p->slot_tiles, 1);
-    k_window_flag<<<w.wf.n, kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf.lo, b.bands, b.rms, b.tile_cnt, b.grp);
-    LAUNCH_CHECK(p);
-    k_tile_prefix<<<w.chain.n, kWfThreads, 0, s>>>(p->d_chain_jobs + w.chain.lo, b.tile_cnt, tile_base, b.n_flagged);
-    LAUNCH_CHECK(p);
-    k_compact<<<(w.wf.n + kWfThreads / 32 - 1) / (kWfThreads / 32), kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf.lo, w.wf.n, b.rms, b.tile_cnt,
-                                                                                          tile_base, b.list, b.grp);
-    LAUNCH_CHECK(p);
-    t_end(p, S_FLAG, s);
-    t_begin(p, S_CHAIN, s);
     const int lanes = chain_lanes(p, w.chain.n);
-    k_att_chain<<<w.chain.n, std::max(lanes, 32), 0, s>>>(p->d_chain_jobs + w.chain.lo, b.list, b.n_flagged, p->d_tables, b.att, p->mb_frames,
-                                            lanes, p->d_chain_stats + 2 * (size_t)w.chain.lo);
-    LAUNCH_CHECK(p);
-    t_end(p, S_CHAIN, s);
-    t_begin(p, S_APPLY, s);
-    k_compress_apply<<<(unsigned)((w.seg_hi - w.seg_lo + 3) / 4), 128, 0, s>>>(p->d_mb_chunks + w.mb_chunks.lo, w.mb_chunks.n, w.seg_lo, w.seg_hi,
-                                                                                b.bands, b.grp, b.att, b.pre, p->mb_frames);
-    LAUNCH_CHECK(p);
-    t_end(p, S_APPLY, s);
-    return AME_OK;
+    int rc = timed(p, S_FLAG, s, [&] {
+        k_window_flag<<<w.wf.n, kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf.lo, b.bands, b.rms, b.tile_cnt, b.grp);
+        if (int rc = launched(p)) return rc;
+        k_tile_prefix<<<w.chain.n, kWfThreads, 0, s>>>(p->d_chain_jobs + w.chain.lo, b.tile_cnt, tile_base, b.n_flagged);
+        if (int rc = launched(p)) return rc;
+        k_compact<<<(w.wf.n + kWfThreads / 32 - 1) / (kWfThreads / 32), kWfThreads, 0, s>>>(p->d_wf_jobs + w.wf.lo, w.wf.n, b.rms, b.tile_cnt,
+                                                                                              tile_base, b.list, b.grp);
+        return launched(p);
+    });
+    if (!rc) rc = timed(p, S_CHAIN, s, [&] {
+        k_att_chain<<<w.chain.n, std::max(lanes, 32), 0, s>>>(p->d_chain_jobs + w.chain.lo, b.list, b.n_flagged, p->d_tables, b.att,
+                                                              p->mb_frames, lanes, p->d_chain_stats + 2 * (size_t)w.chain.lo);
+        return launched(p);
+    });
+    if (!rc) rc = timed(p, S_APPLY, s, [&] {
+        k_compress_apply<<<(unsigned)((w.seg_hi - w.seg_lo + 3) / 4), 128, 0, s>>>(p->d_mb_chunks + w.mb_chunks.lo, w.mb_chunks.n, w.seg_lo,
+                                                                                    w.seg_hi, b.bands, b.grp, b.att, b.pre, p->mb_frames);
+        return launched(p);
+    });
+    return rc;
 }
 
-int run_hist(ame_plan *p, const Wave &w, const int16_t *d_pre, int64_t *d_hist, cudaStream_t s) {
+// K-weighted sub-block energies and sample peaks of `buf` over a k_kweight_energy job table: the input side's
+// (run_hist) or the output meter's (run_meter)
+int launch_kweight(ame_plan *p, const Wave &w, const KwJob *jobs, int n_jobs, const TrackDev *tdev, const int16_t *buf,
+                double *energy, int *peak, cudaStream_t s) {
+    auto *k = w.kw_uni ? k_kweight_energy<true> : k_kweight_energy<false>;
+    k<<<(n_jobs + 127) / 128, 128, 0, s>>>(w.kw_cfg, jobs, n_jobs, p->d_tracks, tdev, buf, energy, peak);
+    return launched(p);
+}
+
+int run_hist(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     const int nt = w.track_hi - w.track_lo;
     if (nt <= 0) return AME_OK;
     CU(cudaMemsetAsync(p->d_peak + w.track_lo, 0, (size_t)nt * 4, s));
-    if (w.kw.n) {
-        t_begin(p, S_KW, s);
-        if (w.kw_uni)
-            k_kweight_energy<true><<<(w.kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_kw_jobs + w.kw.lo, w.kw.n, p->d_tracks, p->d_tdev, d_pre,
-                                                                        p->d_energy, p->d_peak);
-        else
-            k_kweight_energy<false><<<(w.kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_kw_jobs + w.kw.lo, w.kw.n, p->d_tracks, p->d_tdev, d_pre,
-                                                                         p->d_energy, p->d_peak);
-        LAUNCH_CHECK(p);
-        t_end(p, S_KW, s);
-    }
-    t_begin(p, S_TAIL, s);
-    k_tail_peak<<<nt, 128, 0, s>>>(p->d_tracks, p->d_tdev, w.track_lo, w.track_hi, d_pre, p->d_peak);
-    LAUNCH_CHECK(p);
-    t_end(p, S_TAIL, s);
+    int rc = AME_OK;
+    if (w.kw.n)
+        rc = timed(p, S_KW, s, [&] {
+            return launch_kweight(p, w, p->d_kw_jobs + w.kw.lo, w.kw.n, p->d_tdev, b.pre, p->d_energy, p->d_peak, s);
+        });
+    if (!rc) rc = timed(p, S_TAIL, s, [&] {
+        k_tail_peak<<<nt, 128, 0, s>>>(p->d_tracks, p->d_tdev, w.track_lo, w.track_hi, b.pre, p->d_peak);
+        return launched(p);
+    });
+    if (rc) return rc;
     CU(cudaMemsetAsync(p->d_tp + w.track_lo, 0, (size_t)nt * 4, s));
-    if (w.true_peak && w.gain.n) {
-        t_begin(p, S_TP, s);
-        k_true_peak<<<w.gain.n, 256, 0, s>>>(p->d_gain_jobs + w.gain.lo, p->d_tracks, d_pre, p->d_tp);
-        LAUNCH_CHECK(p);
-        t_end(p, S_TP, s);
-    }
-    t_begin(p, S_HIST, s);
-    k_block_hist<<<nt, 256, 0, s>>>(p->d_tdev, w.track_lo, p->d_energy, (long long *)d_hist, p->d_hist_st);
-    LAUNCH_CHECK(p);
-    t_end(p, S_HIST, s);
-    return AME_OK;
+    if (w.true_peak && w.gain.n)
+        rc = timed(p, S_TP, s, [&] {
+            k_true_peak<<<w.gain.n, 256, 0, s>>>(p->d_gain_jobs + w.gain.lo, p->d_tracks, b.pre, p->d_tp);
+            return launched(p);
+        });
+    if (!rc) rc = timed(p, S_HIST, s, [&] {
+        k_block_hist<<<nt, 256, 0, s>>>(p->d_tdev, w.track_lo, p->d_energy, (long long *)b.hist, p->d_hist_st);
+        return launched(p);
+    });
+    return rc;
 }
 
 // static gain (+ the limiter's input and per-tile "last frame over the limit") and the limiter; needs d_results
-int run_apply(ame_plan *p, const Wave &w, const int16_t *d_pre, int16_t *d_out, const Bufs &b, cudaStream_t s) {
-    int16_t *d_norm = b.norm;
-    long long *lim_last = b.lim_last;
+int run_apply(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     if (!w.gain.n) return AME_OK;
-    t_begin(p, S_GAIN, s);
-    if (w.limiter) CU(cudaMemsetAsync(lim_last, 0xff, (size_t)w.lim.n * sizeof(long long), s));      // -1: no frame over the limit
-    k_apply_gain<<<w.gain.n, 256, 0, s>>>(p->d_gain_jobs + w.gain.lo, p->d_results, p->d_tracks, p->d_tdev, d_pre, d_out, d_norm, lim_last);
-    LAUNCH_CHECK(p);
-    t_end(p, S_GAIN, s);
-    if (w.limiter) {
-        t_begin(p, S_LIM, s);
+    int rc = timed(p, S_GAIN, s, [&] {
+        if (w.limiter) CU(cudaMemsetAsync(b.lim_last, 0xff, (size_t)w.lim.n * sizeof(long long), s));   // -1: no frame over the limit
+        k_apply_gain<<<w.gain.n, 256, 0, s>>>(p->d_gain_jobs + w.gain.lo, p->d_results, p->d_tracks, p->d_tdev, b.pre, b.out, b.norm,
+                                              b.lim_last);
+        return launched(p);
+    });
+    if (rc || !w.limiter) return rc;
+    return timed(p, S_LIM, s, [&] {
         const GainJob *gj = p->d_lim_jobs + w.lim.lo;
         constexpr int kLimRounds = 2;                 // repair rounds before the sequential fallback
         int cap = 64;
@@ -388,31 +396,31 @@ int run_apply(ame_plan *p, const Wave &w, const int16_t *d_pre, int16_t *d_out, 
         const size_t smem = lim_smem_bytes(cap);
         for (int round = 0; round <= kLimRounds; ++round) {
             if (round == 0) {                         // the elementwise tiles, 256 threads each
-                k_limiter<<<w.lim.n, 256, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, 0, cap, p->lim_guess);
-                LAUNCH_CHECK(p);
+                k_limiter<<<w.lim.n, 256, smem, s>>>(gj, w.lim.n, b.lim_last, p->d_tracks, b.norm, b.out, b.lim_in, b.lim_out, b.lim_need, 0,
+                                                     cap, p->lim_guess);
+                if (int rc = launched(p)) return rc;
             }
-            k_limiter<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, lim_last, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, round, cap, p->lim_guess);
-            LAUNCH_CHECK(p);
+            k_limiter<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, b.lim_last, p->d_tracks, b.norm, b.out, b.lim_in, b.lim_out, b.lim_need, round,
+                                                cap, p->lim_guess);
+            if (int rc = launched(p)) return rc;
             k_lim_verify<<<(w.lim.n + 3) / 4, 128, 0, s>>>(gj, w.lim.n, p->d_tracks, b.lim_in, b.lim_out, b.lim_need,
                                                              p->d_lim_stats + round);
-            LAUNCH_CHECK(p);
+            if (int rc = launched(p)) return rc;
         }
-        k_lim_fallback<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, p->d_tracks, d_norm, d_out, b.lim_in, b.lim_out, b.lim_need, cap);
-        LAUNCH_CHECK(p);
-        t_end(p, S_LIM, s);
-    }
-    return AME_OK;
+        k_lim_fallback<<<w.lim.n, 32, smem, s>>>(gj, w.lim.n, p->d_tracks, b.norm, b.out, b.lim_in, b.lim_out, b.lim_need, cap);
+        return launched(p);
+    });
 }
 
-int run_gain(ame_plan *p, const Wave &w, const int16_t *d_pre, const int64_t *d_hist, int16_t *d_out, const Bufs &b, cudaStream_t s) {
+int run_gain(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     const int nt = w.track_hi - w.track_lo;
     if (nt <= 0) return AME_OK;
-    t_begin(p, S_FIN, s);
-    k_finalize<<<nt, 128, 0, s>>>(p->d_tracks, w.track_lo, w.track_hi, (const long long *)d_hist, p->d_hist_st, p->d_peak,
-                                             p->d_tp, p->d_results);
-    LAUNCH_CHECK(p);
-    t_end(p, S_FIN, s);
-    return run_apply(p, w, d_pre, d_out, b, s);
+    int rc = timed(p, S_FIN, s, [&] {
+        k_finalize<<<nt, 128, 0, s>>>(p->d_tracks, w.track_lo, w.track_hi, (const long long *)b.hist, p->d_hist_st, p->d_peak, p->d_tp,
+                                      p->d_results);
+        return launched(p);
+    });
+    return rc ? rc : run_apply(p, w, b, s);
 }
 
 // the output meter over the flagged tracks of wave w, read from `buf` (absolute packed-buffer addressing), into `res`
@@ -421,42 +429,35 @@ int run_meter(ame_plan *p, const Wave &w, const int16_t *buf, ame_loudness *res,
     const int nt = w.track_hi - w.track_lo;
     CU(cudaMemsetAsync(p->d_meter_sp + w.track_lo, 0, (size_t)nt * 4, s));
     CU(cudaMemsetAsync(p->d_meter_tp + w.track_lo, 0, (size_t)nt * 4, s));
-    if (w.meter_kw.n) {
-        if (w.kw_uni)
-            k_kweight_energy<true><<<(w.meter_kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_meter_kw + w.meter_kw.lo, w.meter_kw.n, p->d_tracks,
-                                                                              p->d_meter_tdev, buf, p->d_meter_energy, p->d_meter_sp);
-        else
-            k_kweight_energy<false><<<(w.meter_kw.n + 127) / 128, 128, 0, s>>>(w.kw_cfg, p->d_meter_kw + w.meter_kw.lo, w.meter_kw.n, p->d_tracks,
-                                                                               p->d_meter_tdev, buf, p->d_meter_energy, p->d_meter_sp);
-        LAUNCH_CHECK(p);
-    }
+    int rc;
+    if (w.meter_kw.n &&
+        (rc = launch_kweight(p, w, p->d_meter_kw + w.meter_kw.lo, w.meter_kw.n, p->d_meter_tdev, buf, p->d_meter_energy, p->d_meter_sp, s)))
+        return rc;
     if (w.meter_peak.n) {
         k_meter_peak<<<w.meter_peak.n, 256, 0, s>>>(p->d_meter_peak + w.meter_peak.lo, p->d_tracks, buf, p->d_meter_tp, p->d_meter_sp);
-        LAUNCH_CHECK(p);
+        if ((rc = launched(p))) return rc;
     }
     k_meter_finalize<<<w.meter_tracks.n, 256, 0, s>>>(p->d_meter_tracks + w.meter_tracks.lo, p->d_tracks, p->d_meter_tdev, p->d_meter_energy,
                                                       p->d_meter_sp, p->d_meter_tp, res);
-    LAUNCH_CHECK(p);
-    return AME_OK;
+    return launched(p);
 }
 
 int run_measure(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     int rc;
-    if ((rc = run_eq(p, w, b.in, b.pre, s))) return rc;
-    if ((rc = run_split(p, w, b.pre, b.bands, s))) return rc;
+    if ((rc = run_eq(p, w, b, s))) return rc;
+    if ((rc = run_split(p, w, b, s))) return rc;
     if ((rc = run_compress(p, w, b, s))) return rc;
-    return run_hist(p, w, b.pre, b.hist, s);
+    return run_hist(p, w, b, s);
 }
 
 int run_chain_of_stages(ame_plan *p, const Wave &w, const Bufs &b, cudaStream_t s) {
     int rc = run_measure(p, w, b, s);
     if (rc) return rc;
-    return run_gain(p, w, b.pre, b.hist, b.out, b, s);
+    return run_gain(p, w, b, s);
 }
 
 // after a failure in the middle of a pipelined call nothing may still be reading the caller's buffers when we return
-int drain(ame_plan *p, int rc) {
-    (void)p;
+int drain(int rc) {
     if (rc != AME_OK) cudaDeviceSynchronize();
     return rc;
 }
@@ -519,8 +520,8 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
     // ---- layout: tiles are sized for the resident 128-thread CTAs of k_eq and k_band_split -------------
     DeviceShape shape{148, 2, 3};
     cudaDeviceGetAttribute(&shape.n_sm, cudaDevAttrMultiProcessorCount, device);
-    if (p->precision == 1) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shape.occ_eq, k_eq_f32, 128, 0);
-    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shape.occ_eq, k_eq, 128, 0);
+    // 128, not the launch's block size: build_layout counts k_eq's resident threads in 128-thread CTAs (DeviceShape)
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shape.occ_eq, eq_kernel(p).fn, 128, 0);
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shape.occ_split, k_band_split<true>, 128, 0);
     p->n_sm = shape.n_sm;
     JobTables jobs;
@@ -544,6 +545,7 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
         return bail(rc);
     const size_t fb = (size_t)p->total_frames * 4;
     p->slots.resize(p->n_slots);
+    const size_t lim_jobs = std::max(p->slot_lim_jobs, 1);
     for (Slot &sl : p->slots) {
         if ((rc = dmalloc(p, (void **)&sl.pre, (size_t)p->slot_frames * 4)) ||
             (rc = dmalloc(p, (void **)&sl.bands, (size_t)p->mb_frames * 4 * 3)) ||
@@ -556,14 +558,14 @@ int ame_plan_create(int device, const ame_track_params *tracks, int32_t n_tracks
             return bail(rc);
         if (p->any_limiter &&
             ((rc = dmalloc(p, (void **)&sl.norm, (size_t)p->slot_frames * 4)) ||
-             (rc = dmalloc(p, (void **)&sl.lim_last, (size_t)std::max(p->slot_lim_jobs, 1) * sizeof(long long))) ||
-             (rc = dmalloc(p, (void **)&sl.lim_in.st, (size_t)std::max(p->slot_lim_jobs, 1) * sizeof(LimState))) ||
-             (rc = dmalloc(p, (void **)&sl.lim_out.st, (size_t)std::max(p->slot_lim_jobs, 1) * sizeof(LimState))) ||
-             (rc = dmalloc(p, (void **)&sl.lim_in.qframe, (size_t)std::max(p->slot_lim_jobs, 1) * p->lim_keep * sizeof(int))) ||
-             (rc = dmalloc(p, (void **)&sl.lim_out.qframe, (size_t)std::max(p->slot_lim_jobs, 1) * p->lim_keep * sizeof(int))) ||
-             (rc = dmalloc(p, (void **)&sl.lim_in.qdelta, (size_t)std::max(p->slot_lim_jobs, 1) * p->lim_keep * sizeof(double))) ||
-             (rc = dmalloc(p, (void **)&sl.lim_out.qdelta, (size_t)std::max(p->slot_lim_jobs, 1) * p->lim_keep * sizeof(double))) ||
-             (rc = dmalloc(p, (void **)&sl.lim_need, (size_t)std::max(p->slot_lim_jobs, 1) * sizeof(int)))))
+             (rc = dmalloc(p, (void **)&sl.lim_last, lim_jobs * sizeof(long long))) ||
+             (rc = dmalloc(p, (void **)&sl.lim_in.st, lim_jobs * sizeof(LimState))) ||
+             (rc = dmalloc(p, (void **)&sl.lim_out.st, lim_jobs * sizeof(LimState))) ||
+             (rc = dmalloc(p, (void **)&sl.lim_in.qframe, lim_jobs * p->lim_keep * sizeof(int))) ||
+             (rc = dmalloc(p, (void **)&sl.lim_out.qframe, lim_jobs * p->lim_keep * sizeof(int))) ||
+             (rc = dmalloc(p, (void **)&sl.lim_in.qdelta, lim_jobs * p->lim_keep * sizeof(double))) ||
+             (rc = dmalloc(p, (void **)&sl.lim_out.qdelta, lim_jobs * p->lim_keep * sizeof(double))) ||
+             (rc = dmalloc(p, (void **)&sl.lim_need, lim_jobs * sizeof(int)))))
             return bail(rc);
         sl.lim_in.keep = sl.lim_out.keep = p->lim_keep;
         // the filters read a few frames past a track's end (whole 16 / 32-byte groups, never stored): keep them defined
@@ -801,7 +803,9 @@ int ame_stage_eq(ame_plan *p, const int16_t *d_in, int16_t *d_pre, void *stream)
     GUARD(p->device);
     int rc = check_warmth(p);
     if (rc) return rc;
-    return run_eq(p, p->waves[0], d_in, d_pre, (cudaStream_t)stream);
+    Bufs b = start_wave(p, 0, d_in);
+    b.pre = d_pre;
+    return run_eq(p, p->waves[0], b, (cudaStream_t)stream);
 }
 
 int ame_stage_band_split(ame_plan *p, const int16_t *d_pre, int16_t *d_bands, void *stream) {
@@ -809,7 +813,10 @@ int ame_stage_band_split(ame_plan *p, const int16_t *d_pre, int16_t *d_bands, vo
     SINGLE_WAVE(p);
     GUARD(p->device);
     if (p->waves[0].split.n && !d_bands) return fail(AME_E_INVALID, "NULL bands buffer");
-    return run_split(p, p->waves[0], d_pre, d_bands, (cudaStream_t)stream);
+    Bufs b = start_wave(p, 0);
+    b.pre = const_cast<int16_t *>(d_pre);
+    b.bands = d_bands;
+    return run_split(p, p->waves[0], b, (cudaStream_t)stream);
 }
 
 int ame_stage_compress(ame_plan *p, int16_t *d_bands, int16_t *d_pre, void *stream) {
@@ -817,7 +824,7 @@ int ame_stage_compress(ame_plan *p, int16_t *d_bands, int16_t *d_pre, void *stre
     SINGLE_WAVE(p);
     GUARD(p->device);
     if (p->waves[0].chain.n && !d_bands) return fail(AME_E_INVALID, "NULL bands buffer");
-    Bufs b = slot_bufs(p, p->waves[0], nullptr, nullptr);
+    Bufs b = start_wave(p, 0);
     b.bands = d_bands;
     b.pre = d_pre;
     return run_compress(p, p->waves[0], b, (cudaStream_t)stream);
@@ -827,7 +834,10 @@ int ame_stage_loudness_hist(ame_plan *p, const int16_t *d_pre, int64_t *d_hist, 
     if (!p || !d_pre || !d_hist) return fail(AME_E_INVALID, "NULL argument");
     SINGLE_WAVE(p);
     GUARD(p->device);
-    return run_hist(p, p->waves[0], d_pre, d_hist, (cudaStream_t)stream);
+    Bufs b = start_wave(p, 0);
+    b.pre = const_cast<int16_t *>(d_pre);
+    b.hist = d_hist;
+    return run_hist(p, p->waves[0], b, (cudaStream_t)stream);
 }
 
 int ame_stage_apply_gain(ame_plan *p, const int16_t *d_pre, const int64_t *d_hist, int16_t *d_out,
@@ -836,8 +846,10 @@ int ame_stage_apply_gain(ame_plan *p, const int16_t *d_pre, const int64_t *d_his
     SINGLE_WAVE(p);
     GUARD(p->device);
     cudaStream_t s = (cudaStream_t)stream;
-    const Bufs sb = slot_bufs(p, p->waves[0], nullptr, d_out);
-    int rc = run_gain(p, p->waves[0], d_pre, d_hist, d_out, sb, s);
+    Bufs b = start_wave(p, 0, nullptr, d_out);
+    b.pre = const_cast<int16_t *>(d_pre);
+    b.hist = const_cast<int64_t *>(d_hist);
+    int rc = run_gain(p, p->waves[0], b, s);
     if (rc) return rc;
     if (results) {
         CU(cudaMemcpyAsync(results, p->d_results, (size_t)p->n_tracks * sizeof(ame_track_result), cudaMemcpyDeviceToHost, s));
@@ -856,8 +868,9 @@ int ame_stage_limiter(ame_plan *p, const int16_t *d_norm, int16_t *d_out, void *
         if (!(p->tracks[t].flags & AME_F_LIMITER)) return fail(AME_E_INVALID, "track %d has no limiter stage (AME_F_LIMITER)", t);
     cudaStream_t s = (cudaStream_t)stream;
     CU(cudaMemsetAsync(p->d_results, 0, (size_t)p->n_tracks * sizeof(ame_track_result), s));
-    const Bufs sb = slot_bufs(p, p->waves[0], nullptr, d_out);
-    return run_apply(p, p->waves[0], d_norm, d_out, sb, s);
+    Bufs b = start_wave(p, 0, nullptr, d_out);
+    b.pre = const_cast<int16_t *>(d_norm);
+    return run_apply(p, p->waves[0], b, s);
 }
 
 // two-phase form: every wave must keep its pre-normalisation signal between the two calls (n_slots == n_waves)
@@ -865,13 +878,10 @@ int ame_measure_device(ame_plan *p, const int16_t *d_in, int64_t *d_hist, void *
     if (!p || !d_in || !d_hist) return fail(AME_E_INVALID, "NULL argument");
     if (p->slots.size() != p->waves.size()) return fail(AME_E_INVALID, "the two-phase calls need n_slots == n_waves");
     GUARD(p->device);
-    int rc = check_warmth(p);
+    int rc = begin_call(p);
     if (rc) return rc;
-    p->launches = 0;
-    if (p->timing) ++p->t_step;
-    for (size_t w = 0; w < p->waves.size(); ++w) {
-        p->t_wave = (int)std::min<size_t>(w, kMaxTimedWaves - 1);
-        Bufs b = slot_bufs(p, p->waves[w], d_in, nullptr);
+    for (int w = 0; w < (int)p->waves.size(); ++w) {
+        Bufs b = start_wave(p, w, d_in);
         b.hist = d_hist;
         if ((rc = run_measure(p, p->waves[w], b, (cudaStream_t)stream))) return rc;
     }
@@ -884,10 +894,10 @@ int ame_normalize_device(ame_plan *p, const int64_t *d_hist, int16_t *d_out, ame
     GUARD(p->device);
     cudaStream_t s = (cudaStream_t)stream;
     int rc;
-    for (size_t w = 0; w < p->waves.size(); ++w) {
-        p->t_wave = (int)std::min<size_t>(w, kMaxTimedWaves - 1);
-        const Bufs b = slot_bufs(p, p->waves[w], nullptr, d_out);
-        if ((rc = run_gain(p, p->waves[w], b.pre, d_hist, d_out, b, s))) return rc;
+    for (int w = 0; w < (int)p->waves.size(); ++w) {
+        Bufs b = start_wave(p, w, nullptr, d_out);
+        b.hist = const_cast<int64_t *>(d_hist);
+        if ((rc = run_gain(p, p->waves[w], b, s))) return rc;
         if ((rc = run_meter(p, p->waves[w], d_out, p->d_loud_out, s))) return rc;
     }
     if (results) {
@@ -980,34 +990,26 @@ int ame_master_device(ame_plan *p, const int16_t *d_in, int16_t *d_out, ame_trac
     if (!p) return fail(AME_E_INVALID, "NULL plan");
     if (!d_in || !d_out) return fail(AME_E_INVALID, "NULL argument");
     GUARD(p->device);
-    int rc = check_warmth(p);
+    int rc = begin_call(p);
     if (rc) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    const int nw = (int)p->waves.size();
-    p->launches = 0;
-    if (p->timing) ++p->t_step;
-    if (nw <= 1) {
-        p->t_wave = 0;
-        if ((rc = run_chain_of_stages(p, p->waves[0], slot_bufs(p, p->waves[0], d_in, d_out), s))) return rc;
-        if ((rc = run_meter(p, p->waves[0], d_out, p->d_loud_out, s))) return rc;
-    } else {
-        // several waves: fork the caller's stream into the slots' streams and join again.  Waves of different slots
-        // overlap (the latency-bound compressor kernels of one under the FP64-bound filters of another); waves of
-        // one slot follow each other in stream order, which is what recycles the slot.
-        CU(cudaEventRecord(p->ev_in[0], s));
-        const int ns = (int)p->slots.size();
-        for (int w = 0; w < nw; ++w) {
-            cudaStream_t ws = p->slots[p->waves[w].slot].stream;
-            if (w < ns) CU(cudaStreamWaitEvent(ws, p->ev_in[0], 0));
-            p->t_wave = std::min(w, kMaxTimedWaves - 1);
-            if ((rc = run_chain_of_stages(p, p->waves[w], slot_bufs(p, p->waves[w], d_in, d_out), ws))) return drain(p, rc);
-            if ((rc = run_meter(p, p->waves[w], d_out, p->d_loud_out, ws))) return drain(p, rc);
-        }
+    const int nw = (int)p->waves.size(), ns = (int)p->slots.size();
+    // several waves: fork the caller's stream into the slots' streams and join again.  Waves of different slots overlap
+    // (the latency-bound compressor kernels of one under the FP64-bound filters of another); waves of one slot follow
+    // each other in stream order, which is what recycles the slot.  One wave runs on the caller's stream.
+    const bool fork = nw > 1;
+    if (fork) CU(cudaEventRecord(p->ev_in[0], s));
+    for (int w = 0; w < nw; ++w) {
+        cudaStream_t ws = fork ? p->slots[p->waves[w].slot].stream : s;
+        if (fork && w < ns) CU(cudaStreamWaitEvent(ws, p->ev_in[0], 0));
+        if ((rc = run_chain_of_stages(p, p->waves[w], start_wave(p, w, d_in, d_out), ws))) return drain(rc);
+        if ((rc = run_meter(p, p->waves[w], d_out, p->d_loud_out, ws))) return drain(rc);
+    }
+    if (fork)
         for (int k = 0; k < ns; ++k) {
             CU(cudaEventRecord(p->ev_run[k], p->slots[k].stream));
             CU(cudaStreamWaitEvent(s, p->ev_run[k], 0));
         }
-    }
     if (results) {
         CU(cudaMemcpyAsync(results, p->d_results, (size_t)p->n_tracks * sizeof(ame_track_result), cudaMemcpyDeviceToHost, s));
         CU(cudaStreamSynchronize(s));
@@ -1019,10 +1021,8 @@ int ame_master_device(ame_plan *p, const int16_t *d_in, int16_t *d_out, ame_trac
 // events, so the copy engines (PCIe is full duplex) and the SMs work on different waves at the same time.  Pinned host
 // memory makes the copies truly asynchronous; pageable memory still works, the copies then serialise.
 static int master_host_impl(ame_plan *p, const int16_t *h_in, int16_t *h_out, ame_track_result *results) {
-    int rc = check_warmth(p);
+    int rc = begin_call(p);
     if (rc) return rc;
-    p->launches = 0;
-    if (p->timing) ++p->t_step;
     const int nw = (int)p->waves.size();
     const bool tl = p->timing;
     if (tl) {
@@ -1045,8 +1045,7 @@ static int master_host_impl(ame_plan *p, const int16_t *h_in, int16_t *h_out, am
         cudaStream_t ws = p->slots[p->waves[w].slot].stream;
         CU(cudaStreamWaitEvent(ws, p->ev_in[w], 0));
         if (tl) CU(cudaEventRecord(p->tl_ev[2 + 4 * w], ws));
-        p->t_wave = std::min(w, kMaxTimedWaves - 1);
-        if ((rc = run_chain_of_stages(p, p->waves[w], slot_bufs(p, p->waves[w], p->d_in, p->d_out), ws))) return rc;
+        if ((rc = run_chain_of_stages(p, p->waves[w], start_wave(p, w, p->d_in, p->d_out), ws))) return rc;
         CU(cudaEventRecord(p->ev_run[w], ws));
         if (tl) CU(cudaEventRecord(p->tl_ev[3 + 4 * w], ws));
         // the meter reads d_out after ev_run[w]: the wave's D2H copy waits for its kernels, not for its meter
@@ -1106,7 +1105,7 @@ int ame_master_host(ame_plan *p, const int16_t *h_in, int16_t *h_out, ame_track_
     if (!p->d_in || !p->d_out) return fail(AME_E_INVALID, "plan was created without host_io");
     GUARD(p->device);
     // whatever fails in the middle: no copy or kernel may still touch h_in / h_out once we have returned
-    return drain(p, master_host_impl(p, h_in, h_out, results));
+    return drain(master_host_impl(p, h_in, h_out, results));
 }
 
 }  // extern "C"
